@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- alm2map + map2alm wall time on the BASELINE.json configs (default: C4, full-sky CAR 1' IQU, lmax 10800, F64).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--workload C1|C2|C3|C4] [--impl b200|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--workload C1|C2|C3|C4] [--impl b200|reference] [--dump-outputs DIR]
 
 A step = one alm2map followed by one map2alm of the whole IQU (or T) set.  One JSON line is printed by rank 0:
   value   : ms per step, inputs and outputs resident in HBM (device pointers through the C ABI / stage API)
@@ -11,6 +11,10 @@ A step = one alm2map followed by one map2alm of the whole IQU (or T) set.  One J
 N > 1: launched by torchrun, one rank per GPU, m-sharded Legendre + NCCL all-to-all + ring-sharded FFT (strong scaling).
 --impl reference: times that CPU implementation of the reference path (all host threads); the real
 Pixell.jl/libsharp2 cannot run here (no Julia, no libsharp2: DESIGN.md).
+--dump-outputs DIR (one process): after the timed steps, writes what the last one returned -- DIR/map.npy (alm2map
+output, one row per component or batch member) and DIR/alm.npy (map2alm output as (re, im) pairs) -- in the workload's
+float type.  Outputs larger than 32 MB are sampled at positions drawn with a fixed seed from their length alone, so two
+builds run with the same arguments (same seeded inputs) can be compared value for value.
 """
 import argparse
 import ctypes
@@ -248,6 +252,23 @@ def synth_alm_device(torch, nalm, lmax, seed, spin2, device, cdtype):
     return a.to(cdtype).contiguous()
 
 
+DUMP_BYTES = 32 * 10 ** 6     # per dumped file: map.npy + alm.npy stay under 64 MB
+
+
+def dump_outputs(torch, out_dir, name, tensors):
+    """Writes out_dir/<name>.npy: one row per tensor (all of one length), complex values as (re, im) pairs.  When the rows
+    together exceed DUMP_BYTES, each keeps the same positions: a sample drawn with a fixed seed, so it depends on the length alone."""
+    flat = [torch.view_as_real(t).reshape(-1, 2) if t.is_complex() else t.reshape(-1, 1) for t in tensors]
+    n, width = flat[0].shape
+    keep = DUMP_BYTES // (len(flat) * width * flat[0].element_size())
+    if n > keep:
+        idx = torch.from_numpy(np.unique(np.random.default_rng(12345).integers(0, n, keep))).to(flat[0].device)
+        flat = [f.index_select(0, idx) for f in flat]
+    arr = np.stack([f.cpu().numpy() for f in flat])
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, name + ".npy"), arr[:, :, 0] if width == 1 else arr)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -261,11 +282,16 @@ def main():
     ap.add_argument("--no-calibration", action="store_true")
     ap.add_argument("--no-extras", action="store_true")
     ap.add_argument("--no-parity", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs as DIR/map.npy and DIR/alm.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     wl = WORKLOADS[args.workload]
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
+    if args.dump_outputs and (args.impl != "b200" or world > 1):
+        ap.error("--dump-outputs needs the one-process GPU path (--impl b200, one rank)")
     config = {"workload": "%s: %s" % (args.workload, wl["desc"]), "ncomp": wl["ncomp"], "lmax": wl["lmax"],
               "step": "one alm2map + one map2alm", "l2": "inputs larger than L2 (map+alm+phase >> 126 MB)" if args.workload in ("C3", "C4", "C5") else
               "inputs smaller than L2; 256 MB scratch written between timed steps"}
@@ -375,6 +401,9 @@ def main():
             acc[k] = 0 if k in ("n", "launches") else 0.0
         ms_dev = timed(step_dev, 0, args.steps)
         clocks = clk.stop()
+        if args.dump_outputs:
+            dump_outputs(torch, args.dump_outputs, "map", d_map)
+            dump_outputs(torch, args.dump_outputs, "alm", d_out)
         leg_ms, fft_ms = acc["leg"] / acc["n"], acc["fft"] / acc["n"]
         launches = acc["launches"] * args.steps
         stage = {"legendre_ms": leg_ms, "fft_ms": fft_ms}
@@ -747,6 +776,9 @@ def bench_batch(args, wl, config, torch, pixsht, Plan, lib, band, lmax, device, 
     clk = ClockSampler(local_rank); clk.start()
     ms_b = run(batched)
     clocks = clk.stop()
+    if args.dump_outputs:      # before one_by_one() overwrites the buffers
+        dump_outputs(torch, args.dump_outputs, "map", mp)
+        dump_outputs(torch, args.dump_outputs, "alm", out)
     ms_s = run(one_by_one)
     fp64_peak, _ = lib.measure_fma_peak(local_rank)
     # end to end: the same sweep through the host-pointer call on pinned buffers (H2D + D2H inside the timed region)

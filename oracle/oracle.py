@@ -3,9 +3,12 @@
 Two builds of the same source: "ld" (80-bit long double, the parity checker) and "d" (double + OpenMP, the timed CPU
 baseline "port").  Geometry helpers restate src/transforms.jl:33-63 of the reference (ring grid, CC weights x 2pi/nphi).
 """
+import atexit
 import ctypes
 import os
+import shutil
 import subprocess
+import tempfile
 
 import numpy as np
 
@@ -14,9 +17,12 @@ _BUILD = os.path.join(_HERE, "_build")
 
 
 def build(force=False):
-    """(Re)build the oracle shared objects with gcc; no-op when up to date."""
+    """(Re)build the oracle shared objects with gcc; no-op when up to date.  When oracle/_build cannot be written (a
+    read-only tree), a stale or missing build goes to a fresh temporary directory instead."""
+    global _BUILD
     srcs = [os.path.join(_HERE, "sht_oracle.c"), os.path.join(_HERE, "sht_cpu.c")]
-    libs = [os.path.join(_BUILD, "liborc_ld.so"), os.path.join(_BUILD, "liborc_d.so"), os.path.join(_BUILD, "libshtcpu.so")]
+    names = ["liborc_ld.so", "liborc_d.so", "libshtcpu.so"]
+    libs = [os.path.join(_BUILD, n) for n in names]
     fresh = all(os.path.exists(p) and os.path.getmtime(p) >= max(os.path.getmtime(s) for s in srcs) for p in libs)
     # libshtcpu.so is compiled with -march=native: rebuild it when the snapshot travelled to a machine with another CPU
     tag, tag_file = _cpu_tag(), os.path.join(_BUILD, "libshtcpu.host")
@@ -24,11 +30,17 @@ def build(force=False):
         same_host = open(tag_file).read() == tag
     except OSError:
         same_host = False
+    if (force or not fresh or not same_host) and not os.access(_BUILD if os.path.isdir(_BUILD) else _HERE, os.W_OK):
+        _BUILD = tempfile.mkdtemp(prefix="pixsht_oracle_")
+        atexit.register(shutil.rmtree, _BUILD, True)
+        libs = [os.path.join(_BUILD, n) for n in names]
+        tag_file = os.path.join(_BUILD, "libshtcpu.host")
+        fresh = False
     if not same_host and os.path.exists(libs[2]):
         os.remove(libs[2])
         fresh = False
     if force or not fresh:
-        subprocess.check_call(["make", "-C", _HERE, "-s"] + (["-B"] if force else []))
+        subprocess.check_call(["make", "-C", _HERE, "-s", "OUT=" + _BUILD] + (["-B"] if force else []))
     if not same_host:
         with open(tag_file, "w") as f:
             f.write(tag)

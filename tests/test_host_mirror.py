@@ -5,6 +5,8 @@ import ctypes
 import math
 import os
 import re
+import subprocess
+import sys
 
 import numpy as np
 import pytest
@@ -126,16 +128,29 @@ def test_library_exports_every_declared_symbol():
     assert set(_lib.EXPORTS) == decl                  # the ctypes binding knows exactly the declared surface
 
 
+_NO_DEVICE_CHECK = """
+import pixsht
+from pixsht import _lib, fullsky_geometry, sht_band, degree
+lib = _lib.PixshtLib(_lib.DEFAULT_LIB)
+assert lib.device_count() == 0
+shape, wcs = fullsky_geometry(10.0 * degree)
+try:
+    pixsht.Plan(sht_band(shape, wcs), 18)
+except _lib.PixshtError as e:
+    assert e.code == _lib.ERR_NODEVICE and "no CPU fallback" in str(e), e
+else:
+    raise AssertionError("a plan was created without a CUDA device")
+"""
+
+
 def test_library_refuses_to_compute_without_a_device():
     lib = _lib.PixshtLib(_lib.DEFAULT_LIB)
     assert "sm_100a" in lib.version() and "EMULATION" not in lib.version()
     assert int(lib.lib.pixsht_nalm(10800, 10800)) == 58336201
-    if lib.device_count() > 0:
-        pytest.skip("a CUDA device is present: the no-device contract is not observable here")
-    shape, wcs = fullsky_geometry(10.0 * degree)
-    with pytest.raises(_lib.PixshtError) as e:
-        pixsht.Plan(sht_band(shape, wcs), 18)
-    assert e.value.code == _lib.ERR_NODEVICE and "no CPU fallback" in str(e.value)
+    # in a child process that sees no device, also on a machine that has one
+    env = dict(os.environ, CUDA_VISIBLE_DEVICES="", PYTHONPATH=os.pathsep.join([os.path.join(ROOT, "pixell.jl_b200"), ROOT]))
+    r = subprocess.run([sys.executable, "-c", _NO_DEVICE_CHECK], env=env, capture_output=True, text=True, timeout=300)
+    assert r.returncode == 0, r.stderr
 
 
 def test_fejer1_geometry_extension():
