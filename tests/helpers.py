@@ -72,6 +72,9 @@ def oracle_map2alm(m, lmax, mmax=None, spin=0, kind="ld", **kw):
 def oracle_alm2map(alms, shape, wcs, lmax, mmax=None, spin=0, kind="ld", **kw):
     b = pixsht.sht_band(shape, wcs)
     theta, _ = cc_geometry(b.nrings_total, b.nphi, b.ring_first, b.nrings)
+    if kind == "cpu":
+        from oracle import get_cpu_sht
+        return band_to_map(get_cpu_sht().alm2map(alms, theta, b.phi0, b.nphi, lmax, mmax, spin=spin, **kw), b)
     band = get_oracle(kind).alm2map(alms, theta, b.phi0, b.nphi, lmax, mmax, spin=spin, **kw)
     return band_to_map(band, b)
 

@@ -122,8 +122,8 @@ def test_emu_replay_edge_cases(emu_default):
 def test_emu_replay_batched(emu_default):
     import test_gpu_parity as g
     import numpy as np
-    g.test_batched_spin0_equals_single_transforms(6, np.float64, res_deg=10.0, lmax=14)      # groups of 4 + 2
-    g.test_batched_spin0_equals_single_transforms(3, np.float32, res_deg=10.0, lmax=14)      # groups of 2 + 1
+    g.test_batched_spin0_equals_single_transforms(6, np.float64, "host", res_deg=10.0, lmax=14)      # groups of 4 + 2
+    g.test_batched_spin0_equals_single_transforms(3, np.float32, "host", res_deg=10.0, lmax=14)      # groups of 2 + 1
 
 
 def test_emu_replay_multi_gpu_plan(emu_default, monkeypatch):

@@ -416,25 +416,53 @@ def test_c3_size_full_map_against_cpu_port():
 
 
 def test_batch_overlapped_staging_equals_serial(monkeypatch):
-    """Host-pointer batches: the double-buffered staging on the copy streams (the default) gives the same bits as the serial one."""
+    """Host-pointer batches: the double-buffered staging on the copy streams (the default) gives the same bits as the serial one,
+    on pageable arrays (the plan's stager) and on page-locked ones from pixsht_host_alloc (straight to the copy engines)."""
     shape, wcs = fullsky_geometry(8.0 * arcminute)
     lmax = 1350
     band = pixsht.sht_band(shape, wcs)
     alms = [synth_alm(lmax, lmax, 900 + b).astype(np.complex64) for b in range(11)]      # groups 4 + 4 + 2 + 1
-    res = {}
-    for ovl in ("1", "0"):
-        monkeypatch.setenv("PIXSHT_BATCH_OVERLAP", ovl)
-        plan = Plan(band, lmax, dtype=np.float32)
-        maps = plan.alm2map_batch(alms)
-        back = plan.map2alm_batch(maps)
-        res[ovl] = (maps, back)
-        plan.close()
-    for b in range(len(alms)):
-        assert np.array_equal(res["1"][0][b], res["0"][0][b])
-        assert rel_rms(res["1"][1][b], res["0"][1][b]) < 2e-6
-    single = Plan(band, lmax, dtype=np.float32)
-    assert rel_rms(res["1"][0][10], single.alm2map([alms[10]])[0]) < 2e-6
-    single.close()
+    lib = get_lib()
+    for kind in ("pageable", "pinned"):
+        res = {}
+        for ovl in ("1", "0"):
+            monkeypatch.setenv("PIXSHT_BATCH_OVERLAP", ovl)
+            plan = Plan(band, lmax, dtype=np.float32)
+            if kind == "pageable":
+                maps = plan.alm2map_batch(alms)
+                back = plan.map2alm_batch(maps)
+            else:
+                npix = band.nx * band.nrings
+                ptrs = []
+                def pinned(n, dt):
+                    p = ctypes.c_void_p()
+                    lib.check(lib.lib.pixsht_host_alloc(ctypes.byref(p), n * np.dtype(dt).itemsize))
+                    ptrs.append(p.value)
+                    return np.frombuffer((ctypes.c_char * (n * np.dtype(dt).itemsize)).from_address(p.value), dtype=dt)
+                h_alm = [pinned(plan.nalm, np.complex64) for _ in alms]
+                h_map = [pinned(npix, np.float32) for _ in alms]
+                for h, a in zip(h_alm, alms):
+                    h[...] = a
+                for h in h_map:
+                    h[...] = np.nan
+                plan.execute_batch_ptrs(_lib.ALM2MAP, [h.ctypes.data for h in h_alm], [h.ctypes.data for h in h_map], _lib.HOST)
+                for h in h_alm:
+                    h[...] = np.nan
+                plan.execute_batch_ptrs(_lib.MAP2ALM, [h.ctypes.data for h in h_alm], [h.ctypes.data for h in h_map], _lib.HOST)
+                maps = [h.reshape(band.nrings, band.nx).T.copy() for h in h_map]
+                back = [h.copy() for h in h_alm]
+                del h_alm, h_map
+                for p in ptrs:
+                    lib.check(lib.lib.pixsht_host_free(p))
+            res[ovl] = (maps, back)
+            plan.close()
+        for b in range(len(alms)):
+            assert np.array_equal(res["1"][0][b], res["0"][0][b])
+            assert rel_rms(res["1"][1][b], res["0"][1][b]) < 2e-6
+        single = Plan(band, lmax, dtype=np.float32)
+        assert rel_rms(res["1"][0][10], single.alm2map([alms[10]])[0]) < 2e-6
+        assert rel_rms(res["1"][1][10], single.map2alm([res["1"][0][10]])[0]) < 2e-6
+        single.close()
 
 
 def test_host_and_device_paths_agree_and_iqu_is_t_plus_qu():
@@ -873,15 +901,35 @@ def test_fejer1_rings():
     assert rel_rms(map2alm(sub, lmax=30).alm, ref_alm) < 1e-12
 
 
-@pytest.mark.parametrize("nbatch,dtype", [(7, np.float64), (4, np.float64), (3, np.float32)])
-def test_batched_spin0_equals_single_transforms(nbatch, dtype, res_deg=1.0, lmax=180):
+@pytest.mark.parametrize("nbatch,dtype,location", [pytest.param(7, np.float64, "host", id="7-float64"), pytest.param(4, np.float64, "host", id="4-float64"),
+                                                   pytest.param(3, np.float32, "host", id="3-float32")] +
+                         [pytest.param(n, dt, loc, id="%s-%d-%s" % (loc, n, np.dtype(dt).name)) for loc in ("host", "device")
+                          for n, dt in ((1, np.float64), (3, np.float64), (6, np.float32), (9, np.float64))])
+def test_batched_spin0_equals_single_transforms(nbatch, dtype, location, res_deg=1.0, lmax=180):
     """pixsht_execute_batch (groups of 4 / 2 / 1 maps on one recurrence) against the single-map path: synthesis bit for bit
-    (each ring's sum over l is the same sequence of FMAs), analysis to rounding (the cross-lane reduction is grouped differently)."""
+    (each ring's sum over l is the same sequence of FMAs), analysis to rounding (the cross-lane reduction is grouped differently).
+    Batches of 1, 3, 6 and 9 split into groups 1, 2 + 1, 4 + 2 and 4 + 4 + 1: every group size, alone and after another group.
+    location="device": the same batch on device pointers (outputs start as NaN, so a map or alm left unwritten shows)."""
     shape, wcs = fullsky_geometry(res_deg * degree)
     band = pixsht.sht_band(shape, wcs)
     plan = Plan(band, lmax, dtype=dtype)
-    alms = [synth_alm(lmax, lmax, 300 + b) for b in range(nbatch)]
-    maps = plan.alm2map_batch(alms)
+    alms = [synth_alm(lmax, lmax, 300 + b).astype(plan.cdtype) for b in range(nbatch)]
+    rng = np.random.default_rng(8)
+    xs = [np.asfortranarray(rng.standard_normal(shape).astype(dtype)) for _ in range(nbatch)]
+    if location == "host":
+        maps = plan.alm2map_batch(alms)
+        back = plan.map2alm_batch(xs)
+    else:
+        import torch
+        d_alm = [torch.from_numpy(a).cuda() for a in alms]
+        d_map = [torch.full((band.nx * band.nrings,), float("nan"), dtype=getattr(torch, np.dtype(dtype).name), device="cuda") for _ in alms]
+        plan.execute_batch_ptrs(_lib.ALM2MAP, [a.data_ptr() for a in d_alm], [m.data_ptr() for m in d_map], _lib.DEVICE)
+        maps = [m.cpu().numpy().reshape(band.nrings, band.nx).T for m in d_map]
+        d_x = [torch.from_numpy(np.ravel(x, order="F")).cuda() for x in xs]
+        d_out = [torch.full((plan.nalm,), complex("nan+nanj"), dtype=getattr(torch, plan.cdtype.name), device="cuda") for _ in xs]
+        plan.execute_batch_ptrs(_lib.MAP2ALM, [a.data_ptr() for a in d_out], [m.data_ptr() for m in d_x], _lib.DEVICE)
+        back = [a.cpu().numpy() for a in d_out]
+        assert all(np.array_equal(d.cpu().numpy(), np.ravel(x, order="F")) for d, x in zip(d_x, xs))     # inputs untouched
     tol = 1e-13 if dtype == np.float64 else 2e-6
     for b in range(nbatch):
         single = plan.alm2map([alms[b]])[0]
@@ -889,14 +937,11 @@ def test_batched_spin0_equals_single_transforms(nbatch, dtype, res_deg=1.0, lmax
             assert np.array_equal(maps[b], single)
         else:
             assert rel_rms(maps[b], single) < tol
-    rng = np.random.default_rng(8)
-    xs = [np.asfortranarray(rng.standard_normal(shape).astype(dtype)) for _ in range(nbatch)]
-    back = plan.map2alm_batch(xs)
     for b in range(nbatch):
         assert rel_rms(back[b], plan.map2alm([xs[b]])[0]) < tol
     if dtype == np.float64:
-        ref = oracle_map2alm(Enmap(xs[1].astype(np.float64), wcs), lmax)[0]
-        assert rel_rms(back[1], ref) < TOL64
+        ref = oracle_map2alm(Enmap(xs[-1].astype(np.float64), wcs), lmax)[0]
+        assert rel_rms(back[-1], ref) < TOL64
     plan.close()
 
 
