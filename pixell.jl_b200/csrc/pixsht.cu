@@ -1042,9 +1042,13 @@ static void ring_rows(const pixsht_plan* P, int r0, int r1, size_t esz, size_t& 
     off_bytes = (size_t)row0 * P->nx * esz; nbytes = (size_t)(r1 - r0) * P->nx * esz;
 }
 
-// Cumulative work fractions f[0] = 0 < ... < f[K] = 1 of the pieces of the pipelined host path: equal pieces, at most `limit`.
-// (Subdividing the first and the last piece further was measured and changed nothing at C4 / C3: the launches of more and
-// smaller pieces cost what the shorter exposed copies save.)
+// PIXSHT_PIECE_SHAPE=0 makes every pipeline of the host path use equal pieces (read once per process).
+static bool graded_pieces()
+{
+    static const bool on = env_int("PIXSHT_PIECE_SHAPE", 1) != 0;
+    return on;
+}
+
 // Cumulative piece boundaries 0 = f_0 < ... < f_s = 1 of the pipelined host path.  The first piece of an input and the last piece
 // of an output are exposed (nothing runs before the one has arrived / while the other leaves); the pieces in between only have to
 // be short enough for their copy to hide under the neighbouring piece's kernels.
@@ -1053,13 +1057,11 @@ static void ring_rows(const pixsht_plan* P, int r0, int r1, size_t esz, size_t& 
 //            254.7 -> 250.9 ms;
 //   shape 0 (map2alm): equal pieces -- larger middle pieces measured 8 ms of extra gaps in its ring-range inputs, a tapered end
 //            of its alm outputs 1.6 ms more tail (profiles/r02/e2e_probe_pieces*.txt).
-// PIXSHT_PIECE_SHAPE=0 makes every pipeline use equal pieces.
 static std::vector<double> piece_fractions(int nsplit, int limit, int shape = 0)
 {
     std::vector<double> f;
     const int s = std::max(1, std::min(nsplit, limit));
-    static const int allow = env_int("PIXSHT_PIECE_SHAPE", 1);
-    if (shape == 0 || allow == 0 || s < 4) { for (int k = 0; k <= s; ++k) f.push_back((double)k / s); return f; }
+    if (shape == 0 || !graded_pieces() || s < 4) { for (int k = 0; k <= s; ++k) f.push_back((double)k / s); return f; }
     std::vector<double> w(s);
     double tot = 0.0;
     for (int k = 0; k < s; ++k) {
@@ -1070,6 +1072,77 @@ static std::vector<double> piece_fractions(int nsplit, int limit, int shape = 0)
     f.push_back(0.0);
     for (int k = 0; k < s; ++k) { acc += w[k]; f.push_back(k == s - 1 ? 1.0 : acc / tot); }
     return f;
+}
+
+// m boundaries 0 = mb[0] <= ... <= mb[K] = mmax + 1 of equal Legendre work at the cumulative fractions f (work per m ~ lmax - m + 1)
+static std::vector<int> m_bounds(const pixsht_plan* P, const std::vector<double>& f)
+{
+    const int K = (int)f.size() - 1, n = P->mmax + 1;
+    std::vector<int> mb(K + 1);
+    for (int k = 0; k <= K; ++k) mb[k] = (int)std::lround(n * (1.0 - std::sqrt(1.0 - f[k])));
+    mb[0] = 0; mb[K] = n;
+    for (int k = 1; k <= K; ++k) mb[k] = std::max(mb[k], mb[k - 1]);
+    return mb;
+}
+
+// boundaries 0 = cb[0] <= ... <= cb[K] = nch of `nch` ring-pair chunks (pole to equator) of equal Legendre work at the cumulative
+// fractions f (work per pair ~ sin(theta))
+static std::vector<int> chunk_bounds(int nch, const std::vector<double>& f)
+{
+    const int K = (int)f.size() - 1;
+    std::vector<int> cb(K + 1);
+    for (int k = 0; k <= K; ++k) cb[k] = (int)std::lround(nch * (2.0 / 3.14159265358979323846) * std::acos(1.0 - f[k]));
+    cb[0] = 0; cb[K] = nch;
+    for (int k = 1; k <= K; ++k) cb[k] = std::max(cb[k], cb[k - 1]);
+    return cb;
+}
+
+// A piece of the ring pairs: chunks [c0, c1) and the band rings [rings[h][0], rings[h][1]) of their northern (h = 0) and southern
+// members.  A piece of whole components: all chunks, rings {{0, nrings}, {0, 0}}.
+struct Piece { int c0, c1; int rings[2][2]; };
+
+// The pieces between the chunk boundaries cb (chunks of 32 R pairs); false when the pairs of a piece are not contiguous on the sky
+static bool chunk_pieces(const pixsht_plan* P, int R, const std::vector<int>& cb, std::vector<Piece>& pcs)
+{
+    pcs.resize(cb.size() - 1);
+    for (size_t k = 0; k < pcs.size(); ++k) {
+        pcs[k].c0 = cb[k]; pcs[k].c1 = cb[k + 1];
+        if (!pair_range_rings(P, std::min(P->npairs, cb[k] * 32 * R), std::min(P->npairs, cb[k + 1] * 32 * R), pcs[k].rings)) return false;
+    }
+    return true;
+}
+
+// f(r0, r1) for the band-ring range of each hemisphere of a piece that is not empty, north first
+template <class F>
+static int each_hemisphere(const Piece& pc, F&& f)
+{
+    for (int h = 0; h < 2; ++h)
+        if (pc.rings[h][1] > pc.rings[h][0]) { const int rc = f(pc.rings[h][0], pc.rings[h][1]); if (rc) return rc; }
+    return PIXSHT_OK;
+}
+
+// first alm index of column m (nalm past the last column)
+static long long col_begin(const pixsht_plan* P, int m) { return m > P->mmax ? P->nalm : alm_index(P->lmax, m, m); }
+
+// The Float64 alm of component (or batch member) c that the Legendre kernels read and write: `alm` itself in a Float64 plan,
+// the plan's work buffer d_alm64[c] in a Float32 plan.
+static int work_alm(pixsht_plan* P, int c, void* alm, double2** out)
+{
+    if (P->dtype != PIXSHT_F32) { *out = static_cast<double2*>(alm); return PIXSHT_OK; }
+    if (P->d_alm64[c].n < (size_t)P->nalm && P->d_alm64[c].alloc(P->nalm)) return fail(PIXSHT_ERR_NOMEM, "alm work buffer allocation failed");
+    *out = P->d_alm64[c].p;
+    return PIXSHT_OK;
+}
+
+// Float32 plan: converts the alm elements [i0, i1) from the Float32 array `alm` to its work buffer `alm64` (to64) or back, one
+// launch on `st`; nothing in a Float64 plan, whose work buffer is the array
+static void convert_alm(pixsht_plan* P, bool to64, void* alm, double2* alm64, long long i0, long long i1, cudaStream_t st)
+{
+    if (P->dtype != PIXSHT_F32) return;
+    const int grid = P->sm_count > 0 ? P->sm_count * 8 : 256;
+    if (to64) PIXSHT_LAUNCH(k_cvt_f32_to_f64, grid, 256, 0, st, (const float*)alm + 2 * i0, (double*)(alm64 + i0), 2 * (i1 - i0));
+    else PIXSHT_LAUNCH(k_cvt_f64_to_f32, grid, 256, 0, st, (const double*)(alm64 + i0), (float*)alm + 2 * i0, 2 * (i1 - i0));
+    P->launches++;
 }
 
 // every stream of the plan idle, errors swallowed (failure paths: the error text of the original failure is kept by the caller)
@@ -1084,326 +1157,269 @@ static void quiesce(pixsht_plan* P)
     g_err = keep;
 }
 
+// One call of the pipelined host path: its streams, the device staging of each component, whether each of the caller's arrays
+// is pageable (staged by the plan's copy threads) and the dependency events, handed out in order.
+struct HostCall {
+    pixsht_plan* P;
+    int ncomp;
+    void* const* alms; void* const* maps;     // the caller's arrays
+    cudaStream_t sc, sh, sd;                  // compute, host -> device, device -> host
+    size_t esz;
+    void* dmap[3]; void* dalm[3];             // staging, boundary dtype
+    double2* dalm64[3];                       // what the Legendre kernels see
+    bool pg_alm[3], pg_map[3];
+    int ndep;
+    // <= ~45 per call; the batch path recycles entries only after their waits were enqueued
+    cudaEvent_t next_ev() { return P->dep[ndep++ % PIXSHT_NDEP]; }
+    // FFT of components [cb, cb+cn) for band rings [r0, r1)
+    int fft(int dir, int cb, int cn, int r0, int r1)
+    {
+        return stage_fft(P, dir, ncomp, cb, cn, P->d_phase.p + (long long)r0 * ncomp * P->MP, r0, r1 - r0, dmap, sc);
+    }
+    // H2D of the rows of component c for band rings [r0, r1)
+    int rows_in(int c, int r0, int r1)
+    {
+        size_t off, nb; ring_rows(P, r0, r1, esz, off, nb);
+        CU(host_copy_in(P, pg_map[c], (char*)dmap[c] + off, (const char*)maps[c] + off, nb, sh));
+        return PIXSHT_OK;
+    }
+    // FFT + D2H of components [cb, cb+cn) for band rings [r0, r1)
+    int emit_rings(int cb, int cn, int r0, int r1)
+    {
+        int rc = fft(PIXSHT_ALM2MAP, cb, cn, r0, r1); if (rc) return rc;
+        cudaEvent_t e = next_ev();
+        CU(cudaEventRecord(e, sc));
+        CU(cudaStreamWaitEvent(sd, e, 0));
+        size_t off, nb; ring_rows(P, r0, r1, esz, off, nb);
+        for (int c = cb; c < cb + cn; ++c)
+            CU(host_copy_out(P, pg_map[c], (char*)maps[c] + off, (char*)dmap[c] + off, nb, sd));
+        return PIXSHT_OK;
+    }
+    // conversion + D2H of the alm columns of m in [m0, m1) for components [cb, cb+cn)
+    int emit_alm(int cb, int cn, int m0, int m1)
+    {
+        if (m1 <= m0) return PIXSHT_OK;
+        const long long i0 = col_begin(P, m0), i1 = col_begin(P, m1);
+        for (int c = cb; c < cb + cn; ++c) convert_alm(P, false, dalm[c], dalm64[c], i0, i1, sc);
+        cudaEvent_t e = next_ev();
+        CU(cudaEventRecord(e, sc));
+        CU(cudaStreamWaitEvent(sd, e, 0));
+        for (int c = cb; c < cb + cn; ++c)
+            CU(host_copy_out(P, pg_alm[c], (char*)alms[c] + (size_t)i0 * 2 * esz, (char*)dalm[c] + (size_t)i0 * 2 * esz, (size_t)(i1 - i0) * 2 * esz, sd));
+        return PIXSHT_OK;
+    }
+};
+
+static int host_alm2map(HostCall& H)
+{
+    pixsht_plan* P = H.P;
+    cudaStream_t sc = H.sc;
+    const int ncomp = H.ncomp, c0 = ncomp == 3 ? 1 : 0;   // c0: first spin-2 component
+    const bool has0 = ncomp != 2, has2 = ncomp >= 2;
+    const PhaseRef ph = {P->d_phase.p, 0, 0};
+    int rc;
+    // Synthesis of m in [m0, m1) of components [cb, cb+cn) in ring-pair ranges of equal Legendre work, polar side first, so that
+    // the last (exposed) piece of the map copy is the one with the fewest rings; each range's rows leave after its FFT.
+    auto synth_in_ring_pieces = [&](int spin, int cb, int cn, int m0, int m1) -> int {
+        const int R = spin == 0 ? P->R0 : P->R2, nch = leg_total_chunks(P, R);
+        std::vector<Piece> pcs;
+        if (!chunk_pieces(P, R, chunk_bounds(nch, piece_fractions(P->nsplit, nch, 1)), pcs)) pcs.assign(1, {0, nch, {{0, P->nrings}, {0, 0}}});
+        for (const Piece& pc : pcs) {
+            const LegJob J = {spin, ncomp, cb, m0, m1 - m0, nullptr, pc.c0, pc.c1 - pc.c0, ph};
+            int rc2 = synth_launch(P, J, sc); if (rc2) return rc2;
+            rc2 = each_hemisphere(pc, [&](int r0, int r1) { return H.emit_rings(cb, cn, r0, r1); }); if (rc2) return rc2;
+        }
+        return PIXSHT_OK;
+    };
+
+    // input copies: the spin-0 alm goes first, in m ranges of equal Legendre work, so that its synthesis starts after a
+    // fraction of one component has arrived; the polarisation alm follow and arrive under the spin-0 work
+    // A single spin-0 map has no polarisation work for its rows to leave under: its LAST m piece then carries half of the
+    // work and is synthesised in ring ranges whose rows leave one by one (pieces 1 2 4 8 15 thirtieths; tonly_rings).
+    const bool tonly_rings = has0 && !has2 && graded_pieces() && P->nsplit >= 5 && P->mmax + 1 >= 64 && leg_total_chunks(P, P->R0) >= env_int("PIXSHT_TONLY_MINCHUNKS", 16);   // large plans only: the pieces must outweigh their launches
+    const std::vector<int> mb0 = m_bounds(P, tonly_rings ? std::vector<double>{0.0, 1.0 / 30, 3.0 / 30, 7.0 / 30, 15.0 / 30, 1.0}
+                                                         : piece_fractions(P->nsplit, P->mmax + 1, 1));
+    const int K0 = has0 ? (int)mb0.size() - 1 : 0;
+    std::vector<cudaEvent_t> e_t(K0);
+    for (int k = 0; k < K0; ++k) {
+        const long long i0 = col_begin(P, mb0[k]), i1 = col_begin(P, mb0[k + 1]);
+        if (i1 > i0) CU(host_copy_in(P, H.pg_alm[0], (char*)H.dalm[0] + (size_t)i0 * 2 * H.esz, (const char*)H.alms[0] + (size_t)i0 * 2 * H.esz, (size_t)(i1 - i0) * 2 * H.esz, H.sh));
+        e_t[k] = H.next_ev(); CU(cudaEventRecord(e_t[k], H.sh));
+    }
+    cudaEvent_t e_in[3] = {nullptr, nullptr, nullptr};
+    for (int c = (has0 ? 1 : 0); c < ncomp; ++c) {
+        CU(host_copy_in(P, H.pg_alm[c], H.dalm[c], H.alms[c], (size_t)P->nalm * 2 * H.esz, H.sh));
+        e_in[c] = H.next_ev(); CU(cudaEventRecord(e_in[c], H.sh));
+    }
+    if (has0) {
+        rc = ensure_seek(P, 0, sc); if (rc) return rc;
+        for (int k = 0; k < K0; ++k) {
+            const long long i0 = col_begin(P, mb0[k]), i1 = col_begin(P, mb0[k + 1]);
+            CU(cudaStreamWaitEvent(sc, e_t[k], 0));
+            if (i1 <= i0) continue;
+            convert_alm(P, true, H.dalm[0], H.dalm64[0], i0, i1, sc);
+            rc = synth_prep(P, 0, H.dalm64[0], H.dalm64[0], sc, i0, i1 - i0); if (rc) return rc;
+            if (tonly_rings && k == K0 - 1) break;   // the last m piece goes in ring ranges, below
+            const LegJob J = {0, ncomp, 0, mb0[k], mb0[k + 1] - mb0[k], nullptr, 0, leg_total_chunks(P, P->R0), ph};
+            rc = synth_launch(P, J, sc); if (rc) return rc;
+        }
+        rc = tonly_rings ? synth_in_ring_pieces(0, 0, 1, mb0[K0 - 1], mb0[K0]) : H.emit_rings(0, 1, 0, P->nrings); if (rc) return rc;
+    }
+    if (has2) {
+        CU(cudaStreamWaitEvent(sc, e_in[c0], 0));
+        CU(cudaStreamWaitEvent(sc, e_in[c0 + 1], 0));
+        convert_alm(P, true, H.dalm[c0], H.dalm64[c0], 0, P->nalm, sc);
+        convert_alm(P, true, H.dalm[c0 + 1], H.dalm64[c0 + 1], 0, P->nalm, sc);
+        rc = synth_prep(P, 2, H.dalm64[c0], H.dalm64[c0 + 1], sc); if (rc) return rc;
+        rc = synth_in_ring_pieces(2, c0, 2, 0, P->mmax + 1); if (rc) return rc;
+    }
+    return PIXSHT_OK;
+}
+
+static int host_map2alm(HostCall& H)
+{
+    pixsht_plan* P = H.P;
+    cudaStream_t sc = H.sc;
+    const int ncomp = H.ncomp, c0 = ncomp == 3 ? 1 : 0;   // c0: first spin-2 component
+    const bool has0 = ncomp != 2, has2 = ncomp >= 2;
+    const PhaseRef ph = {P->d_phase.p, 0, 0};
+    int rc;
+    // Analysis of chunks [ch0, ch0+nch) of components [cb, cb+cn) in m ranges of equal Legendre work, ascending (the last piece is
+    // the smallest); each range's alm columns leave after its launch.
+    auto anal_in_m_pieces = [&](int spin, int cb, int cn, int ch0, int nch) -> int {
+        const std::vector<int> mb = m_bounds(P, piece_fractions(P->nsplit, P->mmax + 1));
+        for (size_t q = 0; q + 1 < mb.size(); ++q) {
+            const LegJob J = {spin, ncomp, cb, mb[q], mb[q + 1] - mb[q], nullptr, ch0, nch, ph};
+            int rc2 = anal_launch(P, J, H.dalm64[cb], cn == 2 ? H.dalm64[cb + 1] : nullptr, sc); if (rc2) return rc2;
+            rc2 = H.emit_alm(cb, cn, mb[q], mb[q + 1]); if (rc2) return rc2;
+        }
+        return PIXSHT_OK;
+    };
+
+    // input copies: the spin-0 map goes first, in ring-pair ranges (north rows + mirrored south rows), so that its FFTs
+    // and analysis start after a fraction of one component has arrived; the polarisation maps follow
+    const int Ra = P->R0a, nch0 = leg_total_chunks(P, Ra);
+    // The pieces go EQUATOR FIRST (the last of the pole-to-equator chunk ranges is copied and analysed first): the equatorial
+    // chunks carry most of the Legendre work (every m is active there), so the compute stream has a backlog after the first
+    // piece and every later copy hides under it; pole first, the bulk of the spin-0 analysis waited for the end of the whole
+    // component's copy.  Sizes from the equator: 1, 2, 3, 3, ... chunks (the first piece is the exposed head of the call).
+    // PIXSHT_PIECE_SHAPE=0: equal pieces, pole first (round-1 order).
+    const bool eq_first = has0 && graded_pieces() && nch0 >= 4 && P->nsplit >= 4;
+    const bool tonly_m = has0 && !has2 && nch0 >= env_int("PIXSHT_TONLY_MINCHUNKS", 16);   // single spin-0 map of a large plan, see below
+    std::vector<Piece> pcs0;   // in the order they are copied and analysed
+    if (has0) {
+        std::vector<int> cb0;
+        if (eq_first) {
+            cb0.push_back(nch0);
+            for (int k = 0; cb0.back() > 0; ++k) {
+                const int left = cb0.back();
+                int take = (k == 0) ? 1 : (k == 1 ? 2 : std::max(3, (nch0 - 3 + P->nsplit - 3) / std::max(1, P->nsplit - 2)));
+                if ((int)cb0.size() == P->nsplit || take > left) take = left;
+                // a single spin-0 map: the polar 40 % of the chunks (a fifth of the work) stay together as the last piece, which is
+                // analysed in m ranges whose alm columns leave one by one (nothing else would cover that copy)
+                if (tonly_m && k > 0 && nch0 - left >= (nch0 * 3 + 4) / 5) take = left;
+                cb0.push_back(left - take);
+            }
+            std::reverse(cb0.begin(), cb0.end());
+        } else {
+            for (double f : piece_fractions(P->nsplit, nch0)) cb0.push_back((int)std::lround(nch0 * f));
+            cb0.back() = nch0;
+            for (size_t k = 1; k < cb0.size(); ++k) cb0[k] = std::max(cb0[k], cb0[k - 1]);
+        }
+        if (!chunk_pieces(P, Ra, cb0, pcs0)) pcs0.assign(1, {0, nch0, {{0, P->nrings}, {0, 0}}});
+        if (eq_first) std::reverse(pcs0.begin(), pcs0.end());
+    }
+    const int K0 = (int)pcs0.size();
+    std::vector<cudaEvent_t> e_t(K0);
+    for (int k = 0; k < K0; ++k) {
+        rc = each_hemisphere(pcs0[k], [&](int r0, int r1) { return H.rows_in(0, r0, r1); }); if (rc) return rc;
+        e_t[k] = H.next_ev(); CU(cudaEventRecord(e_t[k], H.sh));
+    }
+    // The polarisation maps follow in two parts: the equatorial third of the rings (half of the spin-2 Legendre work), then
+    // the polar rest.  The analysis of the first part (all m) starts as soon as it has arrived -- about when the spin-0 work
+    // ends -- and covers the arrival of the second, which is then analysed in m ranges whose alm columns leave one by one.
+    const int nch2 = leg_total_chunks(P, P->R2a);
+    const int cA = has2 ? (int)std::lround(nch2 * (2.0 / 3.0)) : 0;      // chunks [cA, nch2): the equatorial part
+    std::vector<Piece> parts;                                             // [0]: the polar part, [1]: the equatorial part
+    const bool two_part = has2 && cA > 0 && cA < nch2 && chunk_pieces(P, P->R2a, {0, cA, nch2}, parts);
+    cudaEvent_t e_in[3] = {nullptr, nullptr, nullptr}, e_partA = nullptr;
+    if (two_part) {
+        for (int part : {1, 0}) {
+            for (int c = c0; c < c0 + 2; ++c) {
+                rc = each_hemisphere(parts[part], [&](int r0, int r1) { return H.rows_in(c, r0, r1); }); if (rc) return rc;
+            }
+            cudaEvent_t e = H.next_ev(); CU(cudaEventRecord(e, H.sh));
+            if (part == 1) e_partA = e; else e_in[c0] = e_in[c0 + 1] = e;
+        }
+    } else {
+        for (int c = (has0 ? 1 : 0); c < ncomp; ++c) {
+            CU(host_copy_in(P, H.pg_map[c], H.dmap[c], H.maps[c], (size_t)P->nx * P->ny * H.esz, H.sh));
+            e_in[c] = H.next_ev(); CU(cudaEventRecord(e_in[c], H.sh));
+        }
+    }
+    for (int c = 0; c < ncomp; ++c) CU(cudaMemsetAsync(H.dalm64[c], 0, (size_t)P->nalm * sizeof(double2), sc));
+    if (has0) {
+        // a single spin-0 map: its last (polar) piece is analysed in m ranges, each followed by the copy of its alm columns
+        const bool last_in_m = tonly_m && eq_first && K0 > 1;
+        for (int k = 0; k < K0; ++k) {
+            const Piece& pc = pcs0[k];
+            CU(cudaStreamWaitEvent(sc, e_t[k], 0));
+            rc = each_hemisphere(pc, [&](int r0, int r1) { return H.fft(PIXSHT_MAP2ALM, 0, 1, r0, r1); }); if (rc) return rc;
+            if (last_in_m && k == K0 - 1) rc = anal_in_m_pieces(0, 0, 1, pc.c0, pc.c1 - pc.c0);
+            else {
+                const LegJob J = {0, ncomp, 0, 0, P->mmax + 1, nullptr, pc.c0, pc.c1 - pc.c0, ph};
+                rc = anal_launch(P, J, H.dalm64[0], nullptr, sc);
+            }
+            if (rc) return rc;
+        }
+        if (!last_in_m) { rc = H.emit_alm(0, 1, 0, P->mmax + 1); if (rc) return rc; }
+    }
+    if (has2) {
+        int chunksB = nch2;   // chunks left for the m-range launches below
+        if (two_part) {
+            CU(cudaStreamWaitEvent(sc, e_partA, 0));
+            rc = each_hemisphere(parts[1], [&](int r0, int r1) { return H.fft(PIXSHT_MAP2ALM, c0, 2, r0, r1); }); if (rc) return rc;
+            const LegJob JA = {2, ncomp, c0, 0, P->mmax + 1, nullptr, cA, nch2 - cA, ph};
+            rc = anal_launch(P, JA, H.dalm64[c0], H.dalm64[c0 + 1], sc); if (rc) return rc;
+            chunksB = cA;
+        }
+        CU(cudaStreamWaitEvent(sc, e_in[c0], 0));
+        CU(cudaStreamWaitEvent(sc, e_in[c0 + 1], 0));
+        if (two_part) rc = each_hemisphere(parts[0], [&](int r0, int r1) { return H.fft(PIXSHT_MAP2ALM, c0, 2, r0, r1); });
+        else rc = H.fft(PIXSHT_MAP2ALM, c0, 2, 0, P->nrings);
+        if (rc) return rc;
+        rc = anal_in_m_pieces(2, c0, 2, 0, chunksB); if (rc) return rc;
+    }
+    return PIXSHT_OK;
+}
+
 // Host-pointer transform: copies, Legendre and FFT launches are pipelined over three streams so that most of the PCIe
 // time hides under the Legendre kernels (spin-0 work runs while the polarisation inputs arrive; results leave in
 // split-sized pieces while the next split computes).
 static int execute_host(pixsht_plan* P, int direction, int ncomp, void* const* alms, void* const* maps)
 {
-    cudaStream_t sc = P->stream, sh = P->s_h2d, sd = P->s_d2h;
-    const bool f32 = P->dtype == PIXSHT_F32;
-    const size_t esz = f32 ? 4 : 8;
-    const size_t map_bytes = (size_t)P->nx * P->ny * esz, alm_bytes = (size_t)P->nalm * 2 * esz;
-    const int cvt_grid = P->sm_count > 0 ? P->sm_count * 8 : 256;
-    void* dmap[3] = {nullptr, nullptr, nullptr};
-    void* dalm[3] = {nullptr, nullptr, nullptr};
-    double2* dalm64[3] = {nullptr, nullptr, nullptr};
+    HostCall H = {P, ncomp, alms, maps, P->stream, P->s_h2d, P->s_d2h, P->dtype == PIXSHT_F32 ? sizeof(float) : sizeof(double)};
+    const size_t map_bytes = (size_t)P->nx * P->ny * H.esz, alm_bytes = (size_t)P->nalm * 2 * H.esz;
     for (int c = 0; c < ncomp; ++c) {
         if (P->d_map[c].n < map_bytes && P->d_map[c].alloc(map_bytes)) return fail(PIXSHT_ERR_NOMEM, "map staging allocation failed");
         if (P->d_alm[c].n < alm_bytes && P->d_alm[c].alloc(alm_bytes)) return fail(PIXSHT_ERR_NOMEM, "alm staging allocation failed");
-        dmap[c] = P->d_map[c].p; dalm[c] = P->d_alm[c].p;
-        if (f32) {
-            if (P->d_alm64[c].n < (size_t)P->nalm && P->d_alm64[c].alloc(P->nalm)) return fail(PIXSHT_ERR_NOMEM, "alm work buffer allocation failed");
-            dalm64[c] = P->d_alm64[c].p;
-        } else dalm64[c] = reinterpret_cast<double2*>(dalm[c]);
+        H.dmap[c] = P->d_map[c].p; H.dalm[c] = P->d_alm[c].p;
+        int rc = work_alm(P, c, H.dalm[c], &H.dalm64[c]); if (rc) return rc;
+        H.pg_alm[c] = host_is_pageable(alms[c]); H.pg_map[c] = host_is_pageable(maps[c]);
     }
-    bool pg_alm[3] = {false, false, false}, pg_map[3] = {false, false, false};   // pageable arrays are staged by the plan's copy threads
-    for (int c = 0; c < ncomp; ++c) { pg_alm[c] = host_is_pageable(alms[c]); pg_map[c] = host_is_pageable(maps[c]); }
-    const PhaseRef ph = {P->d_phase.p, 0, 0};
-    int ndep = 0;
-    auto next_ev = [&]() { return P->dep[ndep++ % PIXSHT_NDEP]; };   // <= ~45 per call; the batch path recycles entries only after their waits were enqueued
-    const int c0 = ncomp == 3 ? 1 : 0;          // first spin-2 component
-    const bool has0 = ncomp != 2, has2 = ncomp >= 2;
-    int rc;
 
     // the copy streams start after whatever the caller queued on the compute stream
-    cudaEvent_t e_start = next_ev();
-    CU(cudaEventRecord(e_start, sc));
-    CU(cudaStreamWaitEvent(sh, e_start, 0));
-    CU(cudaStreamWaitEvent(sd, e_start, 0));
-    CU(cudaEventRecord(P->ev[0], sc));
-
-    if (direction == PIXSHT_ALM2MAP) {
-        // input copies: the spin-0 alm goes first, in m ranges of equal Legendre work, so that its synthesis starts after a
-        // fraction of one component has arrived; the polarisation alm follow and arrive under the spin-0 work
-        // A single spin-0 map has no polarisation work for its rows to leave under: its LAST m piece then carries half of the
-        // work and is synthesised in ring ranges whose rows leave one by one (pieces 1 2 4 8 15 thirtieths; tonly_rings below).
-        static const int graded_a2m = env_int("PIXSHT_PIECE_SHAPE", 1);
-        const bool tonly_rings = has0 && !has2 && graded_a2m && P->nsplit >= 5 && P->mmax + 1 >= 64 && leg_total_chunks(P, P->R0) >= env_int("PIXSHT_TONLY_MINCHUNKS", 16);   // large plans only: the pieces must outweigh their launches
-        std::vector<double> f0 = piece_fractions(P->nsplit, P->mmax + 1, 1);
-        if (tonly_rings) f0 = {0.0, 1.0 / 30, 3.0 / 30, 7.0 / 30, 15.0 / 30, 1.0};
-        const int K0 = has0 ? (int)f0.size() - 1 : 0;
-        std::vector<int> mb0(K0 + 1, 0);
-        std::vector<cudaEvent_t> e_t(K0);
-        for (int k = 0; k <= K0; ++k) mb0[k] = (k == K0) ? P->mmax + 1 : (int)std::lround((P->mmax + 1) * (1.0 - std::sqrt(1.0 - f0[k])));
-        for (int k = 1; k <= K0; ++k) mb0[k] = std::max(mb0[k], mb0[k - 1]);
-        auto col0 = [&](int m) { return (m > P->mmax) ? P->nalm : alm_index(P->lmax, m, m); };
-        for (int k = 0; k < K0; ++k) {
-            const long long i0 = col0(mb0[k]), i1 = col0(mb0[k + 1]);
-            if (i1 > i0) CU(host_copy_in(P, pg_alm[0], (char*)dalm[0] + (size_t)i0 * 2 * esz, (const char*)alms[0] + (size_t)i0 * 2 * esz, (size_t)(i1 - i0) * 2 * esz, sh));
-            e_t[k] = next_ev(); CU(cudaEventRecord(e_t[k], sh));
-        }
-        cudaEvent_t e_in[3] = {nullptr, nullptr, nullptr};
-        for (int c = (has0 ? 1 : 0); c < ncomp; ++c) {
-            CU(host_copy_in(P, pg_alm[c], dalm[c], alms[c], alm_bytes, sh));
-            e_in[c] = next_ev(); CU(cudaEventRecord(e_in[c], sh));
-        }
-        auto cvt_in = [&](int c) {
-            if (f32) { PIXSHT_LAUNCH(k_cvt_f32_to_f64, cvt_grid, 256, 0, sc, (const float*)dalm[c], (double*)dalm64[c], 2 * P->nalm); P->launches++; }
-        };
-        // FFT + D2H of components [cb, cb+cn) for band rings [r0, r1)
-        auto emit_rings = [&](int cb, int cn, int r0, int r1) -> int {
-            if (r1 <= r0) return PIXSHT_OK;
-            int rc2 = stage_fft(P, PIXSHT_ALM2MAP, ncomp, cb, cn, P->d_phase.p + (long long)r0 * ncomp * P->MP, r0, r1 - r0, dmap, sc);
-            if (rc2) return rc2;
-            cudaEvent_t e = next_ev();
-            CU(cudaEventRecord(e, sc));
-            CU(cudaStreamWaitEvent(sd, e, 0));
-            size_t off, nb; ring_rows(P, r0, r1, esz, off, nb);
-            for (int c = cb; c < cb + cn; ++c)
-                CU(host_copy_out(P, pg_map[c], (char*)maps[c] + off, (char*)dmap[c] + off, nb, sd));
-            return PIXSHT_OK;
-        };
-        if (has0) {
-            { int rc2 = ensure_seek(P, 0, sc); if (rc2) return rc2; }
-            for (int k = 0; k < K0; ++k) {
-                const long long i0 = col0(mb0[k]), i1 = col0(mb0[k + 1]);
-                CU(cudaStreamWaitEvent(sc, e_t[k], 0));
-                if (i1 <= i0) continue;
-                if (f32) { PIXSHT_LAUNCH(k_cvt_f32_to_f64, cvt_grid, 256, 0, sc, (const float*)dalm[0] + 2 * i0, (double*)(dalm64[0] + i0), 2 * (i1 - i0)); P->launches++; }
-                rc = synth_prep(P, 0, dalm64[0], dalm64[0], sc, i0, i1 - i0); if (rc) return rc;
-                if (tonly_rings && k == K0 - 1) break;   // the last m piece goes in ring ranges, below
-                const LegJob J = {0, ncomp, 0, mb0[k], mb0[k + 1] - mb0[k], nullptr, 0, leg_total_chunks(P, P->R0), ph};
-                rc = synth_launch(P, J, sc); if (rc) return rc;
-            }
-            bool rings_done = false;
-            if (tonly_rings && mb0[K0] > mb0[K0 - 1]) {
-                // ring-pair ranges of equal Legendre work, polar side first: the last (exposed) rows are the fewest
-                const int R = P->R0, nch = leg_total_chunks(P, R);
-                const std::vector<double> fr = piece_fractions(P->nsplit, nch, 1);
-                const int K = (int)fr.size() - 1;
-                std::vector<int> cb(K + 1);
-                for (int k = 0; k <= K; ++k) cb[k] = (int)std::lround(nch * (2.0 / 3.14159265358979323846) * std::acos(1.0 - fr[k]));
-                cb[0] = 0; cb[K] = nch;
-                for (int k = 1; k <= K; ++k) cb[k] = std::max(cb[k], cb[k - 1]);
-                bool ok = true;
-                std::vector<std::array<int, 4>> rr(K);
-                for (int k = 0; k < K && ok; ++k) {
-                    int rng[2][2];
-                    ok = pair_range_rings(P, std::min(P->npairs, cb[k] * 32 * R), std::min(P->npairs, cb[k + 1] * 32 * R), rng);
-                    rr[k] = {rng[0][0], rng[0][1], rng[1][0], rng[1][1]};
-                }
-                if (ok) {
-                    for (int k = 0; k < K; ++k) {
-                        const LegJob J = {0, ncomp, 0, mb0[K0 - 1], mb0[K0] - mb0[K0 - 1], nullptr, cb[k], cb[k + 1] - cb[k], ph};
-                        rc = synth_launch(P, J, sc); if (rc) return rc;
-                        rc = emit_rings(0, 1, rr[k][0], rr[k][1]); if (rc) return rc;
-                        rc = emit_rings(0, 1, rr[k][2], rr[k][3]); if (rc) return rc;
-                    }
-                    rings_done = true;
-                }
-            }
-            if (tonly_rings && !rings_done) {
-                const LegJob J = {0, ncomp, 0, mb0[K0 - 1], mb0[K0] - mb0[K0 - 1], nullptr, 0, leg_total_chunks(P, P->R0), ph};
-                rc = synth_launch(P, J, sc); if (rc) return rc;
-            }
-            if (!rings_done) { rc = emit_rings(0, 1, 0, P->nrings); if (rc) return rc; }
-        }
-        if (has2) {
-            CU(cudaStreamWaitEvent(sc, e_in[c0], 0));
-            CU(cudaStreamWaitEvent(sc, e_in[c0 + 1], 0));
-            cvt_in(c0); cvt_in(c0 + 1);
-            rc = synth_prep(P, 2, dalm64[c0], dalm64[c0 + 1], sc); if (rc) return rc;
-            // splits of the ring pairs with equal Legendre work (work per pair ~ sin(theta)): polar side first, so that
-            // the last (exposed) piece of the map copy is the one with the fewest rings
-            const int R = P->R2, nch = leg_total_chunks(P, R);
-            const std::vector<double> f2 = piece_fractions(P->nsplit, nch, 1);
-            int K = (int)f2.size() - 1;
-            std::vector<int> cb(K + 1);
-            for (int k = 0; k <= K; ++k) cb[k] = (int)std::lround(nch * (2.0 / 3.14159265358979323846) * std::acos(1.0 - f2[k]));
-            cb[0] = 0; cb[K] = nch;
-            for (int k = 1; k <= K; ++k) cb[k] = std::max(cb[k], cb[k - 1]);
-            bool ok = true;
-            std::vector<std::array<int, 4>> rr(K);
-            for (int k = 0; k < K && ok; ++k) {
-                int rng[2][2];
-                ok = pair_range_rings(P, std::min(P->npairs, cb[k] * 32 * R), std::min(P->npairs, cb[k + 1] * 32 * R), rng);
-                rr[k] = {rng[0][0], rng[0][1], rng[1][0], rng[1][1]};
-            }
-            if (!ok) { K = 1; cb = {0, nch}; }
-            for (int k = 0; k < K; ++k) {
-                const LegJob J = {2, ncomp, c0, 0, P->mmax + 1, nullptr, cb[k], cb[k + 1] - cb[k], ph};
-                rc = synth_launch(P, J, sc); if (rc) return rc;
-                if (ok) {
-                    rc = emit_rings(c0, 2, rr[k][0], rr[k][1]); if (rc) return rc;
-                    rc = emit_rings(c0, 2, rr[k][2], rr[k][3]); if (rc) return rc;
-                } else { rc = emit_rings(c0, 2, 0, P->nrings); if (rc) return rc; }
-            }
-        }
-    } else {
-        // input copies: the spin-0 map goes first, in ring-pair ranges (north rows + mirrored south rows), so that its FFTs
-        // and analysis start after a fraction of one component has arrived; the polarisation maps follow
-        const int Ra = P->R0a, nch0 = leg_total_chunks(P, Ra);
-        // The pieces go EQUATOR FIRST (piece K0-1 of the pole-to-equator chunk order is copied and analysed first): the equatorial
-        // chunks carry most of the Legendre work (every m is active there), so the compute stream has a backlog after the first
-        // piece and every later copy hides under it; pole first, the bulk of the spin-0 analysis waited for the end of the whole
-        // component's copy.  Sizes from the equator: 1, 2, 3, 3, ... chunks (the first piece is the exposed head of the call).
-        // PIXSHT_PIECE_SHAPE=0: equal pieces, pole first (round-1 order).
-        static const int graded = env_int("PIXSHT_PIECE_SHAPE", 1);
-        const bool tonly_m = has0 && !has2 && nch0 >= env_int("PIXSHT_TONLY_MINCHUNKS", 16);   // single spin-0 map of a large plan, see below
-        std::vector<int> cb0;
-        int K0 = 0;
-        if (has0 && graded && nch0 >= 4 && P->nsplit >= 4) {
-            std::vector<int> sz;
-            int left = nch0;
-            for (int k = 0; left > 0; ++k) {
-                int take = (k == 0) ? 1 : (k == 1 ? 2 : std::max(3, (nch0 - 3 + P->nsplit - 3) / std::max(1, P->nsplit - 2)));
-                if ((int)sz.size() == P->nsplit - 1 || take > left) take = left;
-                // a single spin-0 map: the polar 40 % of the chunks (a fifth of the work) stay together as the last piece, which is
-                // analysed in m ranges whose alm columns leave one by one (nothing else would cover that copy)
-                if (tonly_m && k > 0 && nch0 - left >= (nch0 * 3 + 4) / 5) take = left;
-                sz.push_back(take); left -= take;
-            }
-            K0 = (int)sz.size();
-            cb0.assign(K0 + 1, 0);
-            for (int k = 0; k < K0; ++k) cb0[K0 - 1 - k] = (k == 0 ? nch0 : cb0[K0 - k]) - sz[k];   // sz[0] = the last (equatorial) interval
-            cb0[K0] = nch0;
-        } else {
-            const std::vector<double> f0 = piece_fractions(P->nsplit, nch0);
-            K0 = has0 ? (int)f0.size() - 1 : 0;
-            cb0.assign(K0 + 1, 0);
-            for (int k = 0; k <= K0; ++k) cb0[k] = (k == K0) ? nch0 : (int)std::lround(nch0 * f0[k]);
-            for (int k = 1; k <= K0; ++k) cb0[k] = std::max(cb0[k], cb0[k - 1]);
-        }
-        const bool eq_first = has0 && graded && nch0 >= 4 && P->nsplit >= 4;
-        std::vector<std::array<int, 4>> rr0(K0);
-        bool ok0 = K0 > 0;
-        for (int k = 0; k < K0 && ok0; ++k) {
-            int rng[2][2];
-            ok0 = pair_range_rings(P, std::min(P->npairs, cb0[k] * 32 * Ra), std::min(P->npairs, cb0[k + 1] * 32 * Ra), rng);
-            rr0[k] = {rng[0][0], rng[0][1], rng[1][0], rng[1][1]};
-        }
-        if (has0 && !ok0) { K0 = 1; cb0 = {0, nch0}; rr0.assign(1, {0, P->nrings, 0, 0}); }
-        std::vector<cudaEvent_t> e_t(K0);
-        for (int kk = 0; kk < K0; ++kk) {
-            const int k = (eq_first && K0 > 1) ? K0 - 1 - kk : kk;
-            for (int h = 0; h < 2; ++h) {
-                if (rr0[k][2 * h + 1] <= rr0[k][2 * h]) continue;
-                size_t off, nb; ring_rows(P, rr0[k][2 * h], rr0[k][2 * h + 1], esz, off, nb);
-                CU(host_copy_in(P, pg_map[0], (char*)dmap[0] + off, (const char*)maps[0] + off, nb, sh));
-            }
-            e_t[k] = next_ev(); CU(cudaEventRecord(e_t[k], sh));
-        }
-        // The polarisation maps follow in two parts: the equatorial third of the rings (half of the spin-2 Legendre work), then
-        // the polar rest.  The analysis of the first part (all m) starts as soon as it has arrived -- about when the spin-0 work
-        // ends -- and covers the arrival of the second, which is then analysed in m ranges whose alm columns leave one by one.
-        const int R2a = P->R2a, nch2 = leg_total_chunks(P, R2a);
-        int cA = has2 ? (int)std::lround(nch2 * (2.0 / 3.0)) : 0;      // chunks [cA, nch2): the equatorial part
-        int rA[2][2] = {{0, 0}, {0, 0}}, rB[2][2] = {{0, 0}, {0, 0}};
-        bool two_part = has2 && cA > 0 && cA < nch2 &&
-                        pair_range_rings(P, std::min(P->npairs, cA * 32 * R2a), P->npairs, rA) && pair_range_rings(P, 0, std::min(P->npairs, cA * 32 * R2a), rB);
-        cudaEvent_t e_in[3] = {nullptr, nullptr, nullptr}, e_partA = nullptr;
-        if (two_part) {
-            for (int part = 0; part < 2; ++part) {
-                for (int c = c0; c < c0 + 2; ++c)
-                    for (int h = 0; h < 2; ++h) {
-                        const int r0 = part == 0 ? rA[h][0] : rB[h][0], r1 = part == 0 ? rA[h][1] : rB[h][1];
-                        if (r1 <= r0) continue;
-                        size_t off, nb; ring_rows(P, r0, r1, esz, off, nb);
-                        CU(host_copy_in(P, pg_map[c], (char*)dmap[c] + off, (const char*)maps[c] + off, nb, sh));
-                    }
-                cudaEvent_t e = next_ev(); CU(cudaEventRecord(e, sh));
-                if (part == 0) e_partA = e; else e_in[c0] = e_in[c0 + 1] = e;
-            }
-        } else {
-            for (int c = (has0 ? 1 : 0); c < ncomp; ++c) {
-                CU(host_copy_in(P, pg_map[c], dmap[c], maps[c], map_bytes, sh));
-                e_in[c] = next_ev(); CU(cudaEventRecord(e_in[c], sh));
-            }
-        }
-        // conversion + D2H of the alm columns of m in [m0, m1) for components [cb, cb+cn)
-        auto emit_alm = [&](int cb, int cn, int m0, int m1) -> int {
-            if (m1 <= m0) return PIXSHT_OK;
-            const long long i0 = alm_index(P->lmax, m0, m0), i1 = (m1 > P->mmax) ? P->nalm : alm_index(P->lmax, m1, m1);
-            if (f32)
-                for (int c = cb; c < cb + cn; ++c) {
-                    PIXSHT_LAUNCH(k_cvt_f64_to_f32, cvt_grid, 256, 0, sc, (const double*)(dalm64[c] + i0), (float*)dalm[c] + 2 * i0, 2 * (i1 - i0));
-                    P->launches++;
-                }
-            cudaEvent_t e = next_ev();
-            CU(cudaEventRecord(e, sc));
-            CU(cudaStreamWaitEvent(sd, e, 0));
-            for (int c = cb; c < cb + cn; ++c)
-                CU(host_copy_out(P, pg_alm[c], (char*)alms[c] + (size_t)i0 * 2 * esz, (char*)dalm[c] + (size_t)i0 * 2 * esz, (size_t)(i1 - i0) * 2 * esz, sd));
-            return PIXSHT_OK;
-        };
-        for (int c = 0; c < ncomp; ++c) CU(cudaMemsetAsync(dalm64[c], 0, (size_t)P->nalm * sizeof(double2), sc));
-        if (has0) {
-            bool t_alm_out = false;
-            for (int kk = 0; kk < K0; ++kk) {
-                const int k = (eq_first && K0 > 1) ? K0 - 1 - kk : kk;
-                CU(cudaStreamWaitEvent(sc, e_t[k], 0));
-                for (int h = 0; h < 2; ++h) {
-                    const int r0 = rr0[k][2 * h], r1 = rr0[k][2 * h + 1];
-                    if (r1 <= r0) continue;
-                    rc = stage_fft(P, PIXSHT_MAP2ALM, ncomp, 0, 1, P->d_phase.p + (long long)r0 * ncomp * P->MP, r0, r1 - r0, dmap, sc); if (rc) return rc;
-                }
-                if (tonly_m && eq_first && K0 > 1 && kk == K0 - 1) {
-                    // last piece of a single spin-0 map: m ranges of equal work, each followed by the copy of its alm columns
-                    const std::vector<double> fm = piece_fractions(P->nsplit, P->mmax + 1);
-                    const int KM = (int)fm.size() - 1;
-                    std::vector<int> mbt(KM + 1);
-                    for (int q = 0; q <= KM; ++q) mbt[q] = (int)std::lround((P->mmax + 1) * (1.0 - std::sqrt(1.0 - fm[q])));
-                    mbt[0] = 0; mbt[KM] = P->mmax + 1;
-                    for (int q = 1; q <= KM; ++q) mbt[q] = std::max(mbt[q], mbt[q - 1]);
-                    for (int q = 0; q < KM; ++q) {
-                        const LegJob J = {0, ncomp, 0, mbt[q], mbt[q + 1] - mbt[q], nullptr, cb0[k], cb0[k + 1] - cb0[k], ph};
-                        rc = anal_launch(P, J, dalm64[0], nullptr, sc); if (rc) return rc;
-                        rc = emit_alm(0, 1, mbt[q], mbt[q + 1]); if (rc) return rc;
-                    }
-                    t_alm_out = true;
-                    continue;
-                }
-                const LegJob J = {0, ncomp, 0, 0, P->mmax + 1, nullptr, cb0[k], cb0[k + 1] - cb0[k], ph};
-                rc = anal_launch(P, J, dalm64[0], nullptr, sc); if (rc) return rc;
-            }
-            if (!t_alm_out) { rc = emit_alm(0, 1, 0, P->mmax + 1); if (rc) return rc; }
-        }
-        if (has2) {
-            int chunksB = nch2;   // chunks left for the m-range launches below
-            if (two_part) {
-                CU(cudaStreamWaitEvent(sc, e_partA, 0));
-                for (int h = 0; h < 2; ++h)
-                    if (rA[h][1] > rA[h][0]) { rc = stage_fft(P, PIXSHT_MAP2ALM, ncomp, c0, 2, P->d_phase.p + (long long)rA[h][0] * ncomp * P->MP, rA[h][0], rA[h][1] - rA[h][0], dmap, sc); if (rc) return rc; }
-                const LegJob JA = {2, ncomp, c0, 0, P->mmax + 1, nullptr, cA, nch2 - cA, ph};
-                rc = anal_launch(P, JA, dalm64[c0], dalm64[c0 + 1], sc); if (rc) return rc;
-                chunksB = cA;
-            }
-            CU(cudaStreamWaitEvent(sc, e_in[c0], 0));
-            CU(cudaStreamWaitEvent(sc, e_in[c0 + 1], 0));
-            if (two_part) {
-                for (int h = 0; h < 2; ++h)
-                    if (rB[h][1] > rB[h][0]) { rc = stage_fft(P, PIXSHT_MAP2ALM, ncomp, c0, 2, P->d_phase.p + (long long)rB[h][0] * ncomp * P->MP, rB[h][0], rB[h][1] - rB[h][0], dmap, sc); if (rc) return rc; }
-            } else {
-                rc = stage_fft(P, PIXSHT_MAP2ALM, ncomp, c0, 2, P->d_phase.p, 0, P->nrings, dmap, sc); if (rc) return rc;
-            }
-            // splits of m with equal Legendre work (work per m ~ lmax - m + 1), ascending: the last piece is the smallest
-            const std::vector<double> f2 = piece_fractions(P->nsplit, P->mmax + 1);
-            const int K = (int)f2.size() - 1;
-            std::vector<int> mb(K + 1);
-            for (int k = 0; k <= K; ++k) mb[k] = (int)std::lround((P->mmax + 1) * (1.0 - std::sqrt(1.0 - f2[k])));
-            mb[0] = 0; mb[K] = P->mmax + 1;
-            for (int k = 1; k <= K; ++k) mb[k] = std::max(mb[k], mb[k - 1]);
-            for (int k = 0; k < K; ++k) {
-                const LegJob J = {2, ncomp, c0, mb[k], mb[k + 1] - mb[k], nullptr, 0, chunksB, ph};
-                rc = anal_launch(P, J, dalm64[c0], dalm64[c0 + 1], sc); if (rc) return rc;
-                rc = emit_alm(c0, 2, mb[k], mb[k + 1]); if (rc) return rc;
-            }
-        }
-    }
-    CU(cudaEventRecord(P->ev[1], sc));
-    CU(cudaStreamSynchronize(sh));
-    CU(cudaStreamSynchronize(sc));
-    CU(cudaStreamSynchronize(sd));
+    cudaEvent_t e_start = H.next_ev();
+    CU(cudaEventRecord(e_start, H.sc));
+    CU(cudaStreamWaitEvent(H.sh, e_start, 0));
+    CU(cudaStreamWaitEvent(H.sd, e_start, 0));
+    CU(cudaEventRecord(P->ev[0], H.sc));
+    const int rc = direction == PIXSHT_ALM2MAP ? host_alm2map(H) : host_map2alm(H);
+    if (rc) return rc;
+    CU(cudaEventRecord(P->ev[1], H.sc));
+    CU(cudaStreamSynchronize(H.sh));
+    CU(cudaStreamSynchronize(H.sc));
+    CU(cudaStreamSynchronize(H.sd));
     CU(cudaGetLastError());
     host_copies_done(P);
     float ms = 0;
@@ -1438,44 +1454,26 @@ extern "C" int pixsht_execute(pixsht_plan* P, int direction, int ncomp, void* co
         return rc;
     }
     cudaStream_t st = P->stream;
-    const bool f32 = P->dtype == PIXSHT_F32;
-    void* dmap[3] = {nullptr, nullptr, nullptr};
-    void* dalm[3] = {nullptr, nullptr, nullptr};     // boundary dtype
     double2* dalm64[3] = {nullptr, nullptr, nullptr}; // what the Legendre kernels see
-    for (int c = 0; c < ncomp; ++c) {
-        dmap[c] = maps[c]; dalm[c] = alms[c];
-        if (f32) {
-            if (P->d_alm64[c].n < (size_t)P->nalm && P->d_alm64[c].alloc(P->nalm)) return fail(PIXSHT_ERR_NOMEM, "alm work buffer allocation failed");
-            dalm64[c] = P->d_alm64[c].p;
-        } else dalm64[c] = reinterpret_cast<double2*>(dalm[c]);
-    }
+    for (int c = 0; c < ncomp; ++c) { rc = work_alm(P, c, alms[c], &dalm64[c]); if (rc) return rc; }
     const PhaseRef ph = {P->d_phase.p, 0, 0};
-    const int cvt_grid = P->sm_count > 0 ? P->sm_count * 8 : 256;
 
     CU(cudaEventRecord(P->ev[0], st));
     CU(cudaEventRecord(P->ev[1], st));
     P->kev_on = true;
     struct KevOff { pixsht_plan* p; ~KevOff() { p->kev_on = false; } } kev_off{P};
     if (direction == PIXSHT_ALM2MAP) {
-        if (f32)
-            for (int c = 0; c < ncomp; ++c) {
-                PIXSHT_LAUNCH(k_cvt_f32_to_f64, cvt_grid, 256, 0, st, (const float*)dalm[c], (double*)dalm64[c], 2 * P->nalm);
-                P->launches++;
-            }
+        for (int c = 0; c < ncomp; ++c) convert_alm(P, true, alms[c], dalm64[c], 0, P->nalm, st);
         rc = stage_alm2phase(P, ncomp, dalm64, P->mmax + 1, nullptr, ph, st); if (rc) return rc;
         CU(cudaEventRecord(P->ev[2], st));
-        rc = stage_fft(P, PIXSHT_ALM2MAP, ncomp, 0, ncomp, P->d_phase.p, 0, P->nrings, dmap, st); if (rc) return rc;
+        rc = stage_fft(P, PIXSHT_ALM2MAP, ncomp, 0, ncomp, P->d_phase.p, 0, P->nrings, maps, st); if (rc) return rc;
         CU(cudaEventRecord(P->ev[3], st));
     } else {
-        rc = stage_fft(P, PIXSHT_MAP2ALM, ncomp, 0, ncomp, P->d_phase.p, 0, P->nrings, dmap, st); if (rc) return rc;
+        rc = stage_fft(P, PIXSHT_MAP2ALM, ncomp, 0, ncomp, P->d_phase.p, 0, P->nrings, maps, st); if (rc) return rc;
         CU(cudaEventRecord(P->ev[2], st));
         for (int c = 0; c < ncomp; ++c) CU(cudaMemsetAsync(dalm64[c], 0, (size_t)P->nalm * sizeof(double2), st));
         rc = stage_phase2alm(P, ncomp, ph, P->mmax + 1, nullptr, dalm64, st); if (rc) return rc;
-        if (f32)
-            for (int c = 0; c < ncomp; ++c) {
-                PIXSHT_LAUNCH(k_cvt_f64_to_f32, cvt_grid, 256, 0, st, (const double*)dalm64[c], (float*)dalm[c], 2 * P->nalm);
-                P->launches++;
-            }
+        for (int c = 0; c < ncomp; ++c) convert_alm(P, false, alms[c], dalm64[c], 0, P->nalm, st);
         CU(cudaEventRecord(P->ev[3], st));
     }
     CU(cudaEventRecord(P->ev[4], st));
@@ -1554,10 +1552,8 @@ static int execute_batch_locked(pixsht_plan* P, int direction, int nbatch, void*
     // the phase rows of a group hold NB "components"; make room for the largest group
     rc = ensure_phase(P, LEG_MAXBATCH); if (rc) return rc;
     cudaStream_t st = P->stream;
-    const bool f32 = P->dtype == PIXSHT_F32;
-    const size_t esz = f32 ? 4 : 8;
+    const size_t esz = P->dtype == PIXSHT_F32 ? 4 : 8;
     const size_t map_bytes = (size_t)P->nx * P->ny * esz, alm_bytes = (size_t)P->nalm * 2 * esz;
-    const int cvt_grid = P->sm_count > 0 ? P->sm_count * 8 : 256;
     // Host pointers: one group of maps is staged, transformed and copied back at a time.  With batch_overlap the staging is double
     // buffered and the copies run on the copy streams, so that group g + 1 arrives and group g - 1 leaves while group g computes.
     const bool ovl = location == PIXSHT_HOST && P->batch_overlap;
@@ -1588,14 +1584,11 @@ static int execute_batch_locked(pixsht_plan* P, int direction, int nbatch, void*
                 if (direction == PIXSHT_ALM2MAP) CU(host_copy_in(P, host_is_pageable(alms[b0 + b]), dalm[b], alms[b0 + b], alm_bytes, sh));
                 else CU(host_copy_in(P, host_is_pageable(maps[b0 + b]), dmap[b], maps[b0 + b], map_bytes, sh));
             } else { dmap[b] = maps[b0 + b]; dalm[b] = alms[b0 + b]; }
-            if (f32) {
-                if (P->d_alm64[k].n < (size_t)P->nalm && P->d_alm64[k].alloc(P->nalm)) return fail(PIXSHT_ERR_NOMEM, "alm work buffer allocation failed");
-                alm64[b] = P->d_alm64[k].p;
-            } else alm64[b] = reinterpret_cast<double2*>(dalm[b]);
+            rc = work_alm(P, k, dalm[b], &alm64[b]); if (rc) return rc;
         }
         if (ovl) { cudaEvent_t e = next_ev(); CU(cudaEventRecord(e, sh)); CU(cudaStreamWaitEvent(st, e, 0)); }
-        if (f32 && direction == PIXSHT_ALM2MAP)
-            for (int b = 0; b < nb; ++b) { PIXSHT_LAUNCH(k_cvt_f32_to_f64, cvt_grid, 256, 0, st, (const float*)dalm[b], (double*)alm64[b], 2 * P->nalm); P->launches++; }
+        if (direction == PIXSHT_ALM2MAP)
+            for (int b = 0; b < nb; ++b) convert_alm(P, true, dalm[b], alm64[b], 0, P->nalm, st);
         if (nb == 4) rc = batch_group<4>(P, direction, alm64, dmap, st);
         else if (nb == 2) rc = batch_group<2>(P, direction, alm64, dmap, st);
         else {
@@ -1612,8 +1605,8 @@ static int execute_batch_locked(pixsht_plan* P, int direction, int nbatch, void*
             }
         }
         if (rc) return rc;
-        if (direction == PIXSHT_MAP2ALM && f32)
-            for (int b = 0; b < nb; ++b) { PIXSHT_LAUNCH(k_cvt_f64_to_f32, cvt_grid, 256, 0, st, (const double*)alm64[b], (float*)dalm[b], 2 * P->nalm); P->launches++; }
+        if (direction == PIXSHT_MAP2ALM)
+            for (int b = 0; b < nb; ++b) convert_alm(P, false, dalm[b], alm64[b], 0, P->nalm, st);
         if (ovl) { cudaEvent_t e = next_ev(); CU(cudaEventRecord(e, st)); CU(cudaStreamWaitEvent(sd, e, 0)); }
         if (location == PIXSHT_HOST) {
             for (int b = 0; b < nb; ++b) {
