@@ -1440,7 +1440,7 @@ extern "C" int pixsht_execute(pixsht_plan* P, int direction, int ncomp, void* co
     if (P->multi) {
         // multi-GPU plan: whole arrays in host memory, or anywhere the GPUs can copy from (the copies use cudaMemcpyDefault)
         const int rcm = execute_multi(P, direction, ncomp, alms, maps, false);
-        if (rcm) { std::string keep = g_err; multi_quiesce(P->multi); g_err = keep; }
+        if (rcm) multi_quiesce(P->multi);
         return rcm;
     }
     int rc = check_device(P->device); if (rc) return rc;
