@@ -101,6 +101,18 @@ int pixsht_host_unregister(void *ptr);
  * Outputs are overwritten (SHARP_ADD is never used by the reference). */
 int pixsht_execute(pixsht_plan *plan, int direction, int ncomp, void *const *alms, void *const *maps, int location);
 
+/* map2alm refined by niter Jacobi iterations, a <- a + A(m - Y a), on one GPU.  niter = 0 is pixsht_execute(MAP2ALM)
+ * exactly.  maps are inputs only and are not modified.  Between iterations the maps, the residual and the alm stay on the
+ * device; with host pointers the maps are copied in once and the alm out once.
+ * (healpy's map2alm(iter=...), python-pixell's map2alm(niter=...).)  The plain analysis is exact on the Clenshaw-Curtis grid
+ * only for lmax <= (nrings-1)/2; above that each iteration removes most of the remaining error, except near the ring's Nyquist
+ * lmax (the columns m << lmax converge slowly there) and on cut-sky bands, which barely improve (DESIGN.md section 10).
+ * ncomp, alms, maps and location as in pixsht_execute; niter < 0 -> PIXSHT_ERR_ARG; a multi-GPU plan with niter > 0 ->
+ * PIXSHT_ERR_UNSUPPORTED.  Device pointers use the plan's stream (or the caller's, pixsht_plan_set_stream) and the call
+ * synchronises it; pixsht_plan_set_polconv applies to the maps and to the residual alike.  The plan keeps ncomp residual
+ * maps of nx*ny elements of its dtype, allocated by the first call with niter > 0. */
+int pixsht_map2alm_iter(pixsht_plan *plan, int ncomp, void *const *alms, void *const *maps, int niter, int location);
+
 /* Batch of nbatch independent spin-0 transforms on one geometry (simulation sweeps; no counterpart in the reference, which
  * transforms one map per libsharp job).  alms[b] / maps[b] as for ncomp = 1.  Up to four maps share one recurrence per
  * (m, ring pair): 2 + 2 NB FP64 ops per (l, m, ring pair) instead of 4 NB. */
@@ -127,7 +139,8 @@ int pixsht_ring_pixarea(const pixsht_geom *geom, double *area /* geom->nrings */
  * device pointers: [1] Legendre stage, [2] FFT stage, [4] whole call (host wall clock), [6] the spin-0 Legendre kernel
  * alone (leg_synth<0,R> or leg_anal<0,R>), [7] the spin-2 Legendre kernel alone;
  * host pointers (copies, Legendre and FFT are pipelined over three streams, so stages overlap): [4] whole call,
- * [5] span of the compute stream; the rest 0 */
+ * [5] span of the compute stream; the rest 0;
+ * pixsht_map2alm_iter with niter > 0 (either location): [4] whole call, [5] span of the compute stream; the rest 0 */
 int pixsht_get_timings(const pixsht_plan *plan, double ms[8]);
 
 /* ---- stage API for the m-sharded multi-GPU pipeline (device pointers, asynchronous on `stream`) ------------

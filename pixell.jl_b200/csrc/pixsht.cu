@@ -119,6 +119,7 @@ struct pixsht_plan {
     DevBuf<double2> d_phase; int phase_ncomp = 0;
     DevBuf<unsigned char> d_map[8], d_alm[8];   // staging of the host paths: components / batch members, two sets for the overlapped batch path
     DevBuf<double2> d_alm64[8];
+    DevBuf<unsigned char> d_resid[3];           // residual maps (plan dtype) of pixsht_map2alm_iter, allocated by its first call with niter > 0
     cudaStream_t stream = nullptr, own_stream = nullptr, s_h2d = nullptr, s_d2h = nullptr;
     cudaEvent_t dep[PIXSHT_NDEP] = {nullptr};   // dependency events of the pipelined host path (at most ~45 per call with 8 splits)
     std::vector<int> h_ringN, h_ringS;
@@ -157,6 +158,29 @@ __global__ void k_cvt_f64_to_f32(const double* __restrict__ in, float* __restric
     long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     const long long step = (long long)gridDim.x * blockDim.x;
     for (; i < n; i += step) out[i] = (float)in[i];
+}
+
+// r <- m - r over the n elements of component blockIdx.y: the residual of the iterative map2alm (m: the caller's maps, r: the
+// maps synthesised from the current alm).  vec: every pointer is 16-byte aligned and the bulk moves in 16-byte loads / stores.
+struct ResidualArgs { const void* m[3]; void* r[3]; };
+template <class T>
+__global__ void __launch_bounds__(256) k_residual(ResidualArgs a, long long n, int vec)
+{
+    constexpr int W = 16 / sizeof(T);
+    struct alignas(16) V { T e[W]; };
+    const int c = blockIdx.y;   // selected, not indexed: an indexed kernel parameter is copied to local memory
+    const T* __restrict__ m = static_cast<const T*>(c == 0 ? a.m[0] : (c == 1 ? a.m[1] : a.m[2]));
+    T* __restrict__ r = static_cast<T*>(c == 0 ? a.r[0] : (c == 1 ? a.r[1] : a.r[2]));
+    const long long i0 = (long long)blockIdx.x * blockDim.x + threadIdx.x, step = (long long)gridDim.x * blockDim.x;
+    const long long nv = vec ? n / W : 0;
+    for (long long i = i0; i < nv; i += step) {
+        const V x = reinterpret_cast<const V*>(m)[i];
+        V y = reinterpret_cast<const V*>(r)[i];
+#pragma unroll
+        for (int j = 0; j < W; ++j) y.e[j] = x.e[j] - y.e[j];
+        reinterpret_cast<V*>(r)[i] = y;
+    }
+    for (long long i = nv * W + i0; i < n; i += step) r[i] = m[i] - r[i];
 }
 
 // the same over the alm columns of the m values m_list[0..nm) (blockIdx.y = position in the list); ZERO: out = 0
@@ -657,6 +681,7 @@ extern "C" void pixsht_plan_destroy(pixsht_plan* P)
     P->d_lg1_hi.release(); P->d_lg1_lo.release(); P->d_ad1.release(); P->d_wg1.release(); P->d_gam1.release(); P->d_rec1.release();
     P->d_lact1.release(); P->d_st1.release();
     for (int c = 0; c < 8; ++c) { P->d_map[c].release(); P->d_alm[c].release(); P->d_alm64[c].release(); }
+    for (auto& r : P->d_resid) r.release();
     for (auto& e : P->ev) if (e) cudaEventDestroy(e);
     for (auto& e : P->kev) if (e) cudaEventDestroy(e);
     for (auto& e : P->dep) if (e) cudaEventDestroy(e);
@@ -1490,6 +1515,101 @@ extern "C" int pixsht_execute(pixsht_plan* P, int direction, int ncomp, void* co
     if (ncomp != 2) { float k; CU(cudaEventElapsedTime(&k, P->kev[0], P->kev[1])); P->timings[6] = k; }
     if (ncomp >= 2) { float k; CU(cudaEventElapsedTime(&k, P->kev[2], P->kev[3])); P->timings[7] = k; }
     return PIXSHT_OK;
+}
+
+// ---------------------------------------------------------------------------------------------------------------
+// iterative map2alm (pixsht_map2alm_iter): a <- A m, then niter times a <- a + A (m - Y a)
+// ---------------------------------------------------------------------------------------------------------------
+// The loop on device pointers, enqueued on `st`: maps (plan dtype) are read only, alms (plan dtype) are written.  The analysis
+// kernels add into the alm, so a <- a + A r is the analysis of r without the memset.  A Float32 plan keeps a in its Float64
+// work alm through every iteration and converts once at the end.
+static int map2alm_iter_device(pixsht_plan* P, int ncomp, void* const* alms, void* const* maps, int niter, cudaStream_t st)
+{
+    const size_t esz = P->dtype == PIXSHT_F32 ? sizeof(float) : sizeof(double);
+    const long long npix = (long long)P->nx * P->ny;
+    double2* a[3] = {nullptr, nullptr, nullptr};
+    void* resid[3] = {nullptr, nullptr, nullptr};
+    ResidualArgs R = {};
+    int vec = 1;
+    for (int c = 0; c < ncomp; ++c) {
+        int rc = work_alm(P, c, alms[c], &a[c]); if (rc) return rc;
+        if (P->d_resid[c].n < (size_t)npix * esz && P->d_resid[c].alloc((size_t)npix * esz)) return fail(PIXSHT_ERR_NOMEM, "residual map allocation failed");
+        resid[c] = R.r[c] = P->d_resid[c].p;
+        R.m[c] = maps[c];
+        if (reinterpret_cast<uintptr_t>(maps[c]) % 16 != 0) vec = 0;
+    }
+    const PhaseRef ph = {P->d_phase.p, 0, 0};
+    int rc = stage_fft(P, PIXSHT_MAP2ALM, ncomp, 0, ncomp, P->d_phase.p, 0, P->nrings, maps, st); if (rc) return rc;
+    for (int c = 0; c < ncomp; ++c) CU(cudaMemsetAsync(a[c], 0, (size_t)P->nalm * sizeof(double2), st));
+    rc = stage_phase2alm(P, ncomp, ph, P->mmax + 1, nullptr, a, st); if (rc) return rc;
+    const dim3 rgrid(P->sm_count > 0 ? P->sm_count * 8 : 256, ncomp);
+    for (int it = 0; it < niter; ++it) {
+        rc = stage_alm2phase(P, ncomp, a, P->mmax + 1, nullptr, ph, st); if (rc) return rc;
+        rc = stage_fft(P, PIXSHT_ALM2MAP, ncomp, 0, ncomp, P->d_phase.p, 0, P->nrings, resid, st); if (rc) return rc;
+        if (P->dtype == PIXSHT_F64) PIXSHT_LAUNCH(k_residual<double>, rgrid, 256, 0, st, R, npix, vec);
+        else PIXSHT_LAUNCH(k_residual<float>, rgrid, 256, 0, st, R, npix, vec);
+        P->launches++;
+        CU(cudaGetLastError());
+        rc = stage_fft(P, PIXSHT_MAP2ALM, ncomp, 0, ncomp, P->d_phase.p, 0, P->nrings, resid, st); if (rc) return rc;
+        rc = stage_phase2alm(P, ncomp, ph, P->mmax + 1, nullptr, a, st); if (rc) return rc;
+    }
+    for (int c = 0; c < ncomp; ++c) convert_alm(P, false, alms[c], a[c], 0, P->nalm, st);
+    return PIXSHT_OK;
+}
+
+// Everything on the compute stream.  Host pointers: the maps go to the plan's map staging once, the loop runs there and the alm
+// come back once, so the iterations see nothing of PCIe.
+static int map2alm_iter_locked(pixsht_plan* P, int ncomp, void* const* alms, void* const* maps, int niter, int location)
+{
+    cudaStream_t st = P->stream;
+    int rc = ensure_phase(P, ncomp); if (rc) return rc;
+    const size_t esz = P->dtype == PIXSHT_F32 ? sizeof(float) : sizeof(double);
+    const size_t map_bytes = (size_t)P->nx * P->ny * esz, alm_bytes = (size_t)P->nalm * 2 * esz;
+    void* dmap[3] = {nullptr, nullptr, nullptr};
+    void* dalm[3] = {nullptr, nullptr, nullptr};
+    if (location == PIXSHT_HOST) {
+        for (int c = 0; c < ncomp; ++c) {
+            if (P->d_map[c].n < map_bytes && P->d_map[c].alloc(map_bytes)) return fail(PIXSHT_ERR_NOMEM, "map staging allocation failed");
+            if (P->d_alm[c].n < alm_bytes && P->d_alm[c].alloc(alm_bytes)) return fail(PIXSHT_ERR_NOMEM, "alm staging allocation failed");
+            dmap[c] = P->d_map[c].p; dalm[c] = P->d_alm[c].p;
+        }
+    }
+    CU(cudaEventRecord(P->ev[0], st));
+    if (location == PIXSHT_HOST) {
+        for (int c = 0; c < ncomp; ++c) CU(host_copy_in(P, host_is_pageable(maps[c]), dmap[c], maps[c], map_bytes, st));
+        rc = map2alm_iter_device(P, ncomp, dalm, dmap, niter, st); if (rc) return rc;
+        for (int c = 0; c < ncomp; ++c) CU(host_copy_out(P, host_is_pageable(alms[c]), alms[c], dalm[c], alm_bytes, st));
+    } else {
+        rc = map2alm_iter_device(P, ncomp, alms, maps, niter, st); if (rc) return rc;
+    }
+    CU(cudaEventRecord(P->ev[1], st));
+    CU(cudaStreamSynchronize(st));
+    CU(cudaGetLastError());
+    host_copies_done(P);
+    float ms = 0;
+    CU(cudaEventElapsedTime(&ms, P->ev[0], P->ev[1]));
+    for (auto& t : P->timings) t = 0;
+    P->timings[5] = ms;
+    return PIXSHT_OK;
+}
+
+extern "C" int pixsht_map2alm_iter(pixsht_plan* P, int ncomp, void* const* alms, void* const* maps, int niter, int location)
+{
+    if (!P || !alms || !maps) return fail(PIXSHT_ERR_ARG, "null argument");
+    if (ncomp < 1 || ncomp > 3) return fail(PIXSHT_ERR_ARG, "SHTs require 1 <= ncomp <= 3, for I, QU, and IQU.");
+    if (location != PIXSHT_HOST && location != PIXSHT_DEVICE) return fail(PIXSHT_ERR_ARG, "bad location");
+    for (int c = 0; c < ncomp; ++c) if (!alms[c] || !maps[c]) return fail(PIXSHT_ERR_ARG, "null component pointer");
+    if (niter < 0) return fail(PIXSHT_ERR_ARG, "niter must be >= 0");
+    if (niter == 0) return pixsht_execute(P, PIXSHT_MAP2ALM, ncomp, alms, maps, location);
+    if (P->multi) return fail(PIXSHT_ERR_UNSUPPORTED, "iterative map2alm (niter > 0) is not supported on a multi-GPU plan");
+    std::lock_guard<std::mutex> lock(P->mu);
+    int rc = check_device(P->device); if (rc) return rc;
+    const auto t_begin = std::chrono::steady_clock::now();
+    P->launches = 0;
+    rc = map2alm_iter_locked(P, ncomp, alms, maps, niter, location);
+    if (rc) quiesce(P);   // nothing may still reference the caller's buffers when a failed call returns
+    P->timings[4] = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_begin).count();
+    return rc;
 }
 
 // ---------------------------------------------------------------------------------------------------------------

@@ -124,6 +124,19 @@ function execute!(p::Plan, dir::Cint, alms::Vector{<:AbstractVector}, maps::Vect
     end
 end
 
+# map2alm refined by `niter` Jacobi iterations, a <- a + A(m - Y a), with the maps, residual and alm kept on the GPU between
+# iterations (pixsht_map2alm_iter; niter = 0 is exactly execute!(p, PIXSHT_MAP2ALM, ...)).  Single-GPU plans only.
+function map2alm_iter!(p::Plan, alms::Vector{<:AbstractVector}, maps::Vector{<:AbstractArray}, niter::Integer)
+    ncomp = length(alms)
+    GC.@preserve alms maps begin
+        aptr = Ptr{Cvoid}[pointer(a) for a in alms]
+        mptr = Ptr{Cvoid}[pointer(m) for m in maps]
+        check(ccall((:pixsht_map2alm_iter, libpixsht), Cint,
+                    (Ptr{Cvoid}, Cint, Ptr{Ptr{Cvoid}}, Ptr{Ptr{Cvoid}}, Cint, Cint),
+                    p.ptr, ncomp, aptr, mptr, niter, PIXSHT_HOST))
+    end
+end
+
 # The reference promotes every map to Float64 before the transform (create_sht_band, src/transforms.jl:71) and returns
 # ComplexF64 alm; so does this binding.  ENV["PIXSHT_F32_BOUNDARY"] = "1" opts in to the Float32-boundary plan for Float32
 # maps (half the PCIe volume, ring FFTs in Float32: ~1e-7 relative, NOT the reference's numerics).
@@ -171,7 +184,7 @@ dense(m::AbstractArray{T}, ::Type{T}) where {T} = is_dense(m) ? m : Array(m)
 dense(m::AbstractArray, ::Type{T}) where {T} = Array{T}(m)
 
 # ---- map2alm: src/transforms.jl:88-165 -------------------------------------------------------------------------
-function _map2alm(maps::Vector, wcs, shape; lmax=nothing, mmax=lmax, polcconv="COSMO")
+function _map2alm(maps::Vector, wcs, shape; lmax=nothing, mmax=lmax, polcconv="COSMO", niter=0)
     if isnothing(lmax)
         lmax = getlmax(wcs); mmax = lmax
     end
@@ -180,28 +193,28 @@ function _map2alm(maps::Vector, wcs, shape; lmax=nothing, mmax=lmax, polcconv="C
     set_polconv!(p, polcconv)
     planes = [dense(m, T) for m in maps]
     alms = [pinned_zeros(Complex{T}, p.nalm) for _ in planes]
-    execute!(p, PIXSHT_MAP2ALM, alms, planes)
+    niter == 0 ? execute!(p, PIXSHT_MAP2ALM, alms, planes) : map2alm_iter!(p, alms, planes, niter)
     [Alm(lmax, mmax, as_complex(a)) for a in alms]
 end
 
-map2alm(m::Enmap{T,2}; lmax=nothing, mmax=lmax) where {T} =
-    _map2alm([parent(m)], getwcs(m), size(m); lmax=lmax, mmax=mmax)[1]
+map2alm(m::Enmap{T,2}; lmax=nothing, mmax=lmax, niter=0) where {T} =
+    _map2alm([parent(m)], getwcs(m), size(m); lmax=lmax, mmax=mmax, niter=niter)[1]
 
-function map2alm(ms::NTuple{2,Enmap{T,2}}; lmax=nothing, mmax=lmax, polcconv="COSMO") where {T}
-    e, b = _map2alm([parent(ms[1]), parent(ms[2])], getwcs(ms[1]), size(ms[1]); lmax=lmax, mmax=mmax, polcconv=polcconv)
+function map2alm(ms::NTuple{2,Enmap{T,2}}; lmax=nothing, mmax=lmax, polcconv="COSMO", niter=0) where {T}
+    e, b = _map2alm([parent(ms[1]), parent(ms[2])], getwcs(ms[1]), size(ms[1]); lmax=lmax, mmax=mmax, polcconv=polcconv, niter=niter)
     (e, b)
 end
 
-function map2alm(ms::NTuple{3,Enmap{T,2}}; lmax=nothing, mmax=lmax, polcconv="COSMO") where {T}
-    t, e, b = _map2alm([parent(m) for m in ms], getwcs(ms[1]), size(ms[1]); lmax=lmax, mmax=mmax, polcconv=polcconv)
+function map2alm(ms::NTuple{3,Enmap{T,2}}; lmax=nothing, mmax=lmax, polcconv="COSMO", niter=0) where {T}
+    t, e, b = _map2alm([parent(m) for m in ms], getwcs(ms[1]), size(ms[1]); lmax=lmax, mmax=mmax, polcconv=polcconv, niter=niter)
     (t, e, b)
 end
 
-function map2alm(m::Enmap{T,3}; lmax=nothing, mmax=lmax, polcconv="COSMO") where {T}
+function map2alm(m::Enmap{T,3}; lmax=nothing, mmax=lmax, polcconv="COSMO", niter=0) where {T}
     ncomp = size(m, 3)
     1 <= ncomp <= 3 || throw(ArgumentError("SHTs require shape (nx,ny,ncomp) with 1 ≤ ncomp ≤ 3, for I, QU, and IQU."))
     planes = [view(parent(m), :, :, c) for c in 1:ncomp]   # contiguous column-major planes: no copy for Array storage
-    out = _map2alm(planes, getwcs(m), size(m)[1:2]; lmax=lmax, mmax=mmax, polcconv=polcconv)
+    out = _map2alm(planes, getwcs(m), size(m)[1:2]; lmax=lmax, mmax=mmax, polcconv=polcconv, niter=niter)
     ncomp == 1 ? out[1] : Tuple(out)
 end
 

@@ -25,7 +25,7 @@ class Geom(ctypes.Structure):
 
 # every symbol include/pixsht.h and include/pixsht_sharp_shim.h declare
 EXPORTS = ["pixsht_plan_create", "pixsht_plan_create_rings", "pixsht_plan_create_multi", "pixsht_multi_shard", "pixsht_execute_sharded",
-           "pixsht_host_alloc", "pixsht_host_free", "pixsht_host_register", "pixsht_host_unregister", "pixsht_plan_destroy", "pixsht_execute", "pixsht_execute_batch", "pixsht_get_timings", "pixsht_plan_set_stream",
+           "pixsht_host_alloc", "pixsht_host_free", "pixsht_host_register", "pixsht_host_unregister", "pixsht_plan_destroy", "pixsht_execute", "pixsht_map2alm_iter", "pixsht_execute_batch", "pixsht_get_timings", "pixsht_plan_set_stream",
            "pixsht_plan_set_stage_families", "pixsht_plan_set_polconv", "pixsht_ring_pixarea", "pixsht_stage_alm2phase", "pixsht_stage_phase2alm", "pixsht_stage_phase2map", "pixsht_stage_map2phase",
            "pixsht_phase_row_len", "pixsht_shared_alloc", "pixsht_shared_open", "pixsht_shared_close", "pixsht_shared_free",
            "pixsht_nalm", "pixsht_alm2cl", "pixsht_plan_info", "pixsht_plan_weights", "pixsht_plan_work", "pixsht_plan_work_per_m", "pixsht_last_error", "pixsht_version",
@@ -59,6 +59,7 @@ class PixshtLib:
         L.pixsht_plan_destroy.argtypes = [vp]
         L.pixsht_plan_destroy.restype = None
         L.pixsht_execute.argtypes = [vp, i32, i32, pvp, pvp, i32]
+        L.pixsht_map2alm_iter.argtypes = [vp, i32, pvp, pvp, i32, i32]
         L.pixsht_execute_batch.argtypes = [vp, i32, i32, pvp, pvp, i32]
         L.pixsht_plan_set_stream.argtypes = [vp, vp, i32]
         L.pixsht_get_timings.argtypes = [vp, ctypes.POINTER(dbl)]

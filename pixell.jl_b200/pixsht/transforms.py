@@ -59,6 +59,11 @@ class Plan:
         self.lib.check(self.lib.lib.pixsht_execute(self.handle, direction, n, _ptr_array(alm_ptrs), _ptr_array(map_ptrs),
                                                    location))
 
+    def map2alm_iter_ptrs(self, alm_ptrs, map_ptrs, niter, location=HOST):
+        """map2alm refined by `niter` Jacobi iterations (pixsht_map2alm_iter); niter = 0 is execute_ptrs(MAP2ALM, ...)."""
+        self.lib.check(self.lib.lib.pixsht_map2alm_iter(self.handle, len(alm_ptrs), _ptr_array(alm_ptrs), _ptr_array(map_ptrs),
+                                                        int(niter), location))
+
     def execute_batch_ptrs(self, direction, alm_ptrs, map_ptrs, location=HOST):
         self.lib.check(self.lib.lib.pixsht_execute_batch(self.handle, direction, len(alm_ptrs), _ptr_array(alm_ptrs), _ptr_array(map_ptrs),
                                                          location))
@@ -128,11 +133,15 @@ class Plan:
         return w, th
 
     # ---- host-array front ends -------------------------------------------------------------------------------
-    def map2alm(self, maps):
-        """maps: list of (nx, ny) Fortran-ordered arrays of the plan dtype (1: T, 2: Q,U, 3: T,Q,U) -> list of alm vectors."""
+    def map2alm(self, maps, niter=0):
+        """maps: list of (nx, ny) Fortran-ordered arrays of the plan dtype (1: T, 2: Q,U, 3: T,Q,U) -> list of alm vectors.
+        niter > 0: the analysis refined by niter Jacobi iterations a <- a + A (m - Y a) on the device (pixsht_map2alm_iter)."""
         maps = [self._as_map(m) for m in maps]
         alms = [np.zeros(self.nalm, dtype=self.cdtype) for _ in maps]
-        self.execute_ptrs(MAP2ALM, [a.ctypes.data for a in alms], [m.ctypes.data for m in maps])
+        if niter == 0:
+            self.execute_ptrs(MAP2ALM, [a.ctypes.data for a in alms], [m.ctypes.data for m in maps])
+        else:
+            self.map2alm_iter_ptrs([a.ctypes.data for a in alms], [m.ctypes.data for m in maps], niter)
         return alms
 
     def alm2map(self, alms):
@@ -220,13 +229,15 @@ def pixareamap_(pixareas, lib=None):
     return pixareas
 
 
-def map2alm(m, lmax=None, mmax=None, lib=None, precision=None, devices=None, polcconv=None):
+def map2alm(m, lmax=None, mmax=None, lib=None, precision=None, devices=None, polcconv=None, niter=0):
     """map2alm(::Enmap{T,2}) / (::NTuple{2}) / (::NTuple{3}) / (::Enmap{T,3})  (src/transforms.jl:88-165).
 
     Returns an Alm (spin 0), or a tuple (E, B) / (T, E, B) of Alm -- the reference's return types; the alm are complex128
     whatever the map's element type, as the reference's (ComplexF64).  precision: see _compute_dtype.  devices: list of GPUs
     for a multi-GPU plan (default: the PIXSHT_DEVICES environment variable, else one GPU).  polcconv: "COSMO" | "IAU", the sign
-    convention of the U map (default: the Enmap's tag from read_map(..., defer_polcconv=True), else COSMO)."""
+    convention of the U map (default: the Enmap's tag from read_map(..., defer_polcconv=True), else COSMO).  niter: Jacobi
+    iterations a <- a + map2alm(m - alm2map(a)) after the plain analysis, as python-pixell's map2alm(niter=...) (single-GPU
+    plans only; they help where lmax exceeds (nrings - 1)/2 of the full-sky grid, DESIGN.md section 10)."""
     if isinstance(m, (tuple, list)):
         maps = list(m)
         if len(maps) not in (2, 3) or any(x.ndim != 2 for x in maps):
@@ -248,7 +259,7 @@ def map2alm(m, lmax=None, mmax=None, lib=None, precision=None, devices=None, pol
     plan = _plan_for(first.shape, first.wcs, lmax, mmax, _compute_dtype(first.dtype, precision), lib, devices)
     # U sign convention of the input: an explicit keyword, else the tag read_map(..., defer_polcconv=True) left on the Enmap
     plan.set_polconv(polcconv if polcconv is not None else getattr(first if not isinstance(m, (tuple, list)) else maps[-1], "polcconv", "COSMO"))
-    alms = [Alm(lmax, mmax, np.asarray(a, dtype=np.complex128)) for a in plan.map2alm(arrays)]
+    alms = [Alm(lmax, mmax, np.asarray(a, dtype=np.complex128)) for a in plan.map2alm(arrays, niter=niter)]
     return alms[0] if len(alms) == 1 else tuple(alms)
 
 
